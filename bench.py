@@ -1,9 +1,14 @@
 #!/usr/bin/env python
 """bench.py — decode tok/s + prefill tok/s for Llama-3-8B bf16, 512-in/128-out (BASELINE.json).
 
-Contract (see the task statement): `python bench.py --gpus N --steps K --warmup W` prints ONE JSON
-line on rank 0.  One "step" = one whole request through the engine: a 512-token prompt is
-prefilled and 128 tokens are decoded greedily (EOS disabled) — BASELINE.json configs[1].
+`python bench.py --gpus N --steps K --warmup W` prints ONE JSON line on rank 0.  One "step" = one
+whole request through the engine: a 512-token prompt is prefilled and 128 tokens are decoded
+greedily (EOS disabled) — BASELINE.json configs[1].  K steps are timed, after W untimed ones.
+
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step returned to its caller:
+one [batch, 128] float64 array per token-event field, DIR/<field>.npy (token_id, index,
+finish_reason, prompt_tokens, completion_tokens; the wall-clock t_ms is left out).  Prompts and
+weights are seeded, so two builds run with the same arguments can be compared array for array.
 
   value        decode tok/s from CUDA-event time of the decode steps (inputs resident in HBM)
   prefill      prefill tok/s from CUDA-event time of the prefill steps (+ tensor roofline)
@@ -42,6 +47,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 PROMPT, GEN = 512, 128
 PARITY_TOL_CPU = 0.30    # margin to the fp32 CPU oracle's arg-max logit (logit std ~1.3 at 8B; bf16 activations): the near-tie bound of
@@ -118,6 +124,17 @@ class ClockSampler:
 def make_prompt(i, vocab, n=PROMPT):
     import numpy as np
     return np.random.RandomState(1000 + i).randint(0, vocab, n).astype("int32").tolist()
+
+
+DUMP_FIELDS = ("token_id", "index", "finish_reason", "prompt_tokens", "completion_tokens")
+
+
+def dump_outputs(out_dir, requests):
+    """requests: per request, the token events the engine returned -> out_dir/<field>.npy, float64 [requests, events]."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for f in DUMP_FIELDS:
+        np.save(os.path.join(out_dir, f + ".npy"), np.array([[e[f] for e in evs] for evs in requests], dtype=np.float64))
 
 
 # ------------------------------------------------------------------------------ CPU arms ----
@@ -366,6 +383,7 @@ def run_ours(args):
         sampler.start()
     t0 = time.perf_counter()
     first_to_last_ms, n_dec_tokens, req_tps, req_ms = 0.0, 0, [], []
+    toks = []
     for i in range(args.steps):
         toks, _ = run_requests([make_prompt(i * args.batch + j, model["vocab"]) for j in range(args.batch)], GEN)
         lo, hi = [], []
@@ -379,6 +397,8 @@ def run_ours(args):
     torch.cuda.synchronize()
     wall = time.perf_counter() - t0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, toks)
     h1 = eng.health()
     d = lambda k: h1[k] - h0[k]
     vals = torch.tensor([d("gpu_ms_decode"), d("gpu_ms_prefill"), wall * 1e3, first_to_last_ms, sum(req_ms)],
@@ -523,6 +543,7 @@ def main():
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=5)
     ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the token events of the last timed step as DIR/<field>.npy")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--model", default="8b", choices=["8b", "tiny"])
     ap.add_argument("--batch", type=int, default=1, help="concurrent streams per step of the main leg (1 = BASELINE configs[1])")
@@ -547,6 +568,8 @@ def main():
                           "kind": "port", "sample": rq["sample"]}))
         return
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs needs --impl ours")
         run_reference(args)
     else:
         run_ours(args)
