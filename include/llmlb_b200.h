@@ -75,16 +75,16 @@ typedef struct llmlb_engine_config {
   uint64_t synthetic_seed;   /* weights are generated on-device from this seed (see
                                 llmlb_engine_load_tensor to overwrite with real ones) */
   uint32_t use_cuda_graphs;  /* capture decode steps per batch width */
-  uint32_t gemm_impl;        /* 0 = tcgen05/TMEM/TMA tiles (default), 1 = mma.sync tiles */
+  uint32_t gemm_impl;        /* must be 0 (tcgen05/TMEM/TMA tiles); anything else: LLMLB_E_INVALID_ARG */
   uint32_t lookahead;        /* decode steps in flight before the host reads tokens (0 = 2) */
   /* Back-pressure, mirroring the gateway's own queue (llmlb/src/config.rs:80-99, QueueConfig) and its
    * per-request inference timeout (llmlb/src/types/endpoint.rs:389).  0 = no limit. */
   uint32_t queue_max;          /* waiting requests beyond this: submit returns LLMLB_E_QUEUE_FULL (gateway: 429) */
   uint32_t queue_timeout_ms;   /* a request still waiting for admission after this finishes QUEUE_TIMEOUT (504) */
   uint32_t request_timeout_ms; /* a request not finished this long after submit finishes DEADLINE (504 timeout) */
-  uint32_t attn_impl;          /* prefill attention: 0 = tcgen05 + TMEM + TMA (default), 1 = mma.sync baseline */
-  uint32_t tp_proto;           /* tensor-parallel decode exchange: bit 0: 0 = {value, epoch} pairs (default), 1 = values + flags;
-                                  bit 1: 1 = owner CTAs fold the partials and the consumer grid gathers the result through L2 */
+  uint32_t attn_impl;          /* must be 0 (prefill attention on tcgen05 + TMEM + TMA); anything else: LLMLB_E_INVALID_ARG */
+  uint32_t tp_proto;           /* must be 0 (tensor-parallel decode exchange of {value, epoch} pairs); anything else:
+                                  LLMLB_E_INVALID_ARG */
   uint32_t reserved[3];
 } llmlb_engine_config;
 
@@ -239,15 +239,10 @@ int llmlb_op_rope_table(float* table, uint32_t max_pos, float theta, void* strea
 int llmlb_op_rope_append(void* qkv_bf16, const int32_t* positions, const int32_t* page_of_token,
                          const float* rope_table, void* k_pages, void* v_pages, uint32_t n_tokens,
                          uint32_t n_heads, uint32_t n_kv_heads, void* stream);
-/* a2.6 causal GQA prefill attention over paged K/V.  tiles: int32[n_tiles][4] =
- * {first q row in qkv, q rows in tile (<=64), position of first row, row into block_tables}. */
-int llmlb_op_prefill_attention(const void* qkv_bf16, const void* k_pages, const void* v_pages,
-                               const int32_t* block_tables, uint32_t bt_stride,
-                               const int32_t* tiles, uint32_t n_tiles, void* out_bf16,
-                               uint32_t n_heads, uint32_t n_kv_heads, void* stream);
-/* a2.6 on the 5th-generation tensor cores (tcgen05.mma, S and PV in TMEM, Q/K/V staged by TMA; V is
- * consumed MN-major straight from its [token][d] pages).  Same contract as above with q tiles of up to
- * 128 rows; k_pages / v_pages are ONE layer's pool [n_pages][n_kv][64][128]; n_tokens = rows of qkv. */
+/* a2.6 causal GQA prefill attention over paged K/V on the 5th-generation tensor cores (tcgen05.mma, S and
+ * PV in TMEM, Q/K/V staged by TMA; V is consumed MN-major straight from its [token][d] pages).
+ * tiles: int32[n_tiles][4] = {first q row in qkv, q rows in tile (<=128), position of first row, row into
+ * block_tables}; k_pages / v_pages are ONE layer's pool [n_pages][n_kv][64][128]; n_tokens = rows of qkv. */
 int llmlb_op_prefill_attention_tc(const void* qkv_bf16, uint32_t n_tokens, const void* k_pages,
                                   const void* v_pages, uint32_t n_pages, const int32_t* block_tables,
                                   uint32_t bt_stride, const int32_t* tiles, uint32_t n_tiles,

@@ -5,11 +5,12 @@
 // RoPE uses a precomputed fp32 (cos,sin) table [position][64] (HF rotate-half pairing i, i+64).
 //
 //  * rope_append_kernel       prefill: rotate q,k in place in the qkv activation, write k,v pages
-//  * prefill_attention_kernel causal GQA flash attention, mma.sync m16n8k16 bf16, 64-row q tiles,
-//                             K/V pages staged with cp.async (double-buffered), fp32 softmax
+//                             (prefill attention itself runs on tcgen05: attention_tc.cu)
 //  * decode_attention_kernel  one new token per sequence: rotate q,k, append k,v, split-KV
 //                             attention over the pages (HBM-bound: ctx*2*128*2 B per kv head),
-//                             last-arriving CTA merges the splits
+//                             the cluster leader merges the splits through DSMEM
+//  * decode_attention_mma_kernel  wide batches, no split: one warp per (sequence, head group),
+//                             mma.sync m16n8k16 over K/V staged by cp.async
 #include "../../include/llmlb_b200.h"
 #include "common.cuh"
 
@@ -73,7 +74,7 @@ rope_append_kernel(__nv_bfloat16* __restrict__ qkv, const int32_t* __restrict__ 
   }
 }
 
-// ------------------------------------------------------------------ prefill attention -------
+// ------------------------------------------------------------------ mma.sync / cp.async / DSMEM helpers ---
 __device__ __forceinline__ void cp_async16(void* smem, const void* gmem, bool valid) {
   uint32_t s = (uint32_t)__cvta_generic_to_shared(smem);
   int sz = valid ? 16 : 0;
@@ -140,189 +141,6 @@ __device__ __forceinline__ void st_dsmem_f4(uint32_t ra, float4 v) {
 }
 __device__ __forceinline__ void st_dsmem_f32(uint32_t ra, float v) {
   asm volatile("st.shared::cluster.f32 [%0], %1;" ::"r"(ra), "f"(v) : "memory");
-}
-
-constexpr int kPfRows = 64;  // q rows per CTA
-constexpr int kPfThreads = 128;
-
-__global__ void __launch_bounds__(kPfThreads)
-prefill_attention_kernel(const __nv_bfloat16* __restrict__ qkv,
-                         const __nv_bfloat16* __restrict__ k_pages,
-                         const __nv_bfloat16* __restrict__ v_pages,
-                         const int32_t* __restrict__ block_tables, uint32_t bt_stride,
-                         const int4* __restrict__ tiles, __nv_bfloat16* __restrict__ out,
-                         uint32_t n_heads, uint32_t n_kv) {
-  extern __shared__ __align__(128) uint8_t smem_raw[];
-  __nv_bfloat16* sq = reinterpret_cast<__nv_bfloat16*>(smem_raw);   // 64 x 128
-  __nv_bfloat16* sk = sq + kPfRows * kHeadDim;                      // 2 x 64 x 128
-  __nv_bfloat16* sv = sk + 2 * kPageTokens * kHeadDim;              // 2 x 64 x 128
-
-  const int4 tile = tiles[blockIdx.x];
-  const uint32_t q_row0 = tile.x, n_rows = tile.y, pos0 = tile.z, bt_row = tile.w;
-  const uint32_t head = blockIdx.y, kvh = head / (n_heads / n_kv);
-  const uint32_t width = (n_heads + 2 * n_kv) * kHeadDim;
-  const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const uint32_t g = lane >> 2, t4 = lane & 3;
-  const int32_t* bt = block_tables + size_t(bt_row) * bt_stride;
-  const uint32_t kv_len = pos0 + n_rows;                   // causal horizon of this tile
-  const uint32_t n_kv_tiles = (kv_len + kPageTokens - 1) / kPageTokens;
-
-  auto load_kv = [&](uint32_t kt, uint32_t buf) {
-    const int32_t page = bt[kt];
-    const __nv_bfloat16* kg = k_pages + (size_t(page) * n_kv + kvh) * kPageTokens * kHeadDim;
-    const __nv_bfloat16* vg = v_pages + (size_t(page) * n_kv + kvh) * kPageTokens * kHeadDim;
-    __nv_bfloat16* dk = sk + buf * kPageTokens * kHeadDim;
-    __nv_bfloat16* dv = sv + buf * kPageTokens * kHeadDim;
-#pragma unroll
-    for (uint32_t i = 0; i < 8; ++i) {
-      uint32_t c = tid + i * kPfThreads;  // 1024 chunks
-      uint32_t r = c >> 4, ch = c & 15;
-      bool valid = kt * kPageTokens + r < kv_len;
-      cp_async16(dk + swz(r, ch), kg + r * kHeadDim + ch * 8, valid);
-      cp_async16(dv + swz(r, ch), vg + r * kHeadDim + ch * 8, valid);
-    }
-  };
-
-  // Q tile -> smem (rows past n_rows are zero-filled)
-#pragma unroll
-  for (uint32_t i = 0; i < 8; ++i) {
-    uint32_t c = tid + i * kPfThreads;
-    uint32_t r = c >> 4, ch = c & 15;
-    bool valid = r < n_rows;
-    const __nv_bfloat16* src =
-        qkv + size_t(q_row0 + (valid ? r : 0)) * width + size_t(head) * kHeadDim + ch * 8;
-    cp_async16(sq + swz(r, ch), src, valid);
-  }
-  load_kv(0, 0);
-  cp_async_commit();
-
-  uint32_t qf[8][4];
-  float o[16][4];
-#pragma unroll
-  for (int i = 0; i < 16; ++i) o[i][0] = o[i][1] = o[i][2] = o[i][3] = 0.f;
-  float m_run[2] = {-INFINITY, -INFINITY}, l_run[2] = {0.f, 0.f};
-  const float scale = rsqrtf(float(kHeadDim)) * kLog2e;
-
-  for (uint32_t kt = 0; kt < n_kv_tiles; ++kt) {
-    const uint32_t buf = kt & 1;
-    if (kt + 1 < n_kv_tiles) load_kv(kt + 1, buf ^ 1);
-    cp_async_commit();
-    cp_async_wait<1>();
-    __syncthreads();
-    if (kt == 0) {
-#pragma unroll
-      for (int ks = 0; ks < 8; ++ks) {
-        uint32_t m = lane >> 3;
-        uint32_t r = warp * 16 + (lane & 7) + (m & 1) * 8;
-        uint32_t ch = ks * 2 + (m >> 1);
-        ldmatrix_x4(qf[ks], sq + swz(r, ch));
-      }
-    }
-    const __nv_bfloat16* tk = sk + buf * kPageTokens * kHeadDim;
-    const __nv_bfloat16* tv = sv + buf * kPageTokens * kHeadDim;
-
-    // S = Q K^T  (16 x 64 per warp)
-    float s[8][4];
-#pragma unroll
-    for (int nb = 0; nb < 8; ++nb) {
-      s[nb][0] = s[nb][1] = s[nb][2] = s[nb][3] = 0.f;
-#pragma unroll
-      for (int kp = 0; kp < 4; ++kp) {  // two k-steps per ldmatrix.x4
-        uint32_t kb[4];
-        uint32_t m = lane >> 3;
-        uint32_t r = nb * 8 + (lane & 7);
-        uint32_t ch = kp * 4 + m;
-        ldmatrix_x4(kb, tk + swz(r, ch));
-        mma_bf16_16816(s[nb], qf[kp * 2], kb[0], kb[1]);
-        mma_bf16_16816(s[nb], qf[kp * 2 + 1], kb[2], kb[3]);
-      }
-    }
-    // scale, causal mask, online softmax
-    const uint32_t kv0 = kt * kPageTokens;
-    const bool need_mask = kv0 + kPageTokens > pos0 + warp * 16 + 1;  // conservative
-    float m_new[2] = {m_run[0], m_run[1]};
-#pragma unroll
-    for (int nb = 0; nb < 8; ++nb) {
-#pragma unroll
-      for (int e = 0; e < 4; ++e) {
-        float v = s[nb][e] * scale;
-        if (need_mask) {
-          uint32_t kvp = kv0 + nb * 8 + t4 * 2 + (e & 1);
-          uint32_t qp = pos0 + warp * 16 + g + (e >> 1) * 8;
-          if (kvp > qp) v = -INFINITY;
-        }
-        s[nb][e] = v;
-        m_new[e >> 1] = fmaxf(m_new[e >> 1], v);
-      }
-    }
-#pragma unroll
-    for (int h = 0; h < 2; ++h) {
-      m_new[h] = fmaxf(m_new[h], __shfl_xor_sync(0xffffffffu, m_new[h], 1));
-      m_new[h] = fmaxf(m_new[h], __shfl_xor_sync(0xffffffffu, m_new[h], 2));
-    }
-    float corr[2], rsum[2] = {0.f, 0.f};
-#pragma unroll
-    for (int h = 0; h < 2; ++h) {
-      float mu = (m_new[h] == -INFINITY) ? 0.f : m_new[h];
-      corr[h] = exp2f(m_run[h] - mu);  // m_run=-inf -> 0
-      m_run[h] = m_new[h];
-#pragma unroll
-      for (int nb = 0; nb < 8; ++nb) {
-        float p0 = exp2f(s[nb][h * 2] - mu), p1 = exp2f(s[nb][h * 2 + 1] - mu);
-        s[nb][h * 2] = p0;
-        s[nb][h * 2 + 1] = p1;
-        rsum[h] += p0 + p1;
-      }
-      l_run[h] = l_run[h] * corr[h] + rsum[h];
-    }
-#pragma unroll
-    for (int nb = 0; nb < 16; ++nb) {
-      o[nb][0] *= corr[0]; o[nb][1] *= corr[0];
-      o[nb][2] *= corr[1]; o[nb][3] *= corr[1];
-    }
-    // O += P V : P (16 x 64) as A fragments, 4 k-steps of 16 tokens
-#pragma unroll
-    for (int ks = 0; ks < 4; ++ks) {
-      uint32_t pa[4];
-      pa[0] = pack_bf16(s[2 * ks][0], s[2 * ks][1]);
-      pa[1] = pack_bf16(s[2 * ks][2], s[2 * ks][3]);
-      pa[2] = pack_bf16(s[2 * ks + 1][0], s[2 * ks + 1][1]);
-      pa[3] = pack_bf16(s[2 * ks + 1][2], s[2 * ks + 1][3]);
-#pragma unroll
-      for (int np = 0; np < 8; ++np) {  // two 8-wide d blocks per ldmatrix.x4.trans
-        uint32_t vb[4];
-        uint32_t m = lane >> 3;
-        uint32_t r = ks * 16 + (m & 1) * 8 + (lane & 7);
-        uint32_t ch = np * 2 + (m >> 1);
-        ldmatrix_x4_trans(vb, tv + swz(r, ch));
-        mma_bf16_16816(o[np * 2], pa, vb[0], vb[1]);
-        mma_bf16_16816(o[np * 2 + 1], pa, vb[2], vb[3]);
-      }
-    }
-    __syncthreads();  // all warps done with buf before it is refilled
-  }
-  cp_async_wait<0>();
-
-  // finalize: row sums across the 4 lanes of a quad, write bf16
-#pragma unroll
-  for (int h = 0; h < 2; ++h) {
-    l_run[h] += __shfl_xor_sync(0xffffffffu, l_run[h], 1);
-    l_run[h] += __shfl_xor_sync(0xffffffffu, l_run[h], 2);
-  }
-  const uint32_t out_w = n_heads * kHeadDim;
-#pragma unroll
-  for (int h = 0; h < 2; ++h) {
-    uint32_t r = warp * 16 + g + h * 8;
-    if (r < n_rows) {
-      float inv = 1.f / l_run[h];
-      __nv_bfloat16* dst = out + size_t(q_row0 + r) * out_w + size_t(head) * kHeadDim;
-#pragma unroll
-      for (int nb = 0; nb < 16; ++nb) {
-        uint32_t v = pack_bf16(o[nb][h * 2] * inv, o[nb][h * 2 + 1] * inv);
-        *reinterpret_cast<uint32_t*>(dst + nb * 8 + t4 * 2) = v;
-      }
-    }
-  }
 }
 
 // ------------------------------------------------------------------ decode attention --------
@@ -623,7 +441,7 @@ int rope_append_launch(void* qkv, const int32_t* positions, const int32_t* page_
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = (pdl && !(g_dbg_no_pdl & 16u)) ? 1 : 0;
+  cfg.numAttrs = pdl ? 1 : 0;
   LLMLB_CUDA_CHECK(cudaLaunchKernelEx(&cfg, rope_append_kernel, (__nv_bfloat16*)qkv, positions, page_of_token,
                                       (const float2*)rope_table, (__nv_bfloat16*)k_pages, (__nv_bfloat16*)v_pages, n_heads, n_kv,
                                       pdl ? 1u : 0u));
@@ -642,32 +460,6 @@ extern "C" int llmlb_op_rope_append(void* qkv, const int32_t* positions,
   }
   return rope_append_launch(qkv, positions, page_of_token, rope_table, k_pages, v_pages, n_tokens, n_heads, n_kv, false,
                             (cudaStream_t)stream);
-}
-
-extern "C" int llmlb_op_prefill_attention(const void* qkv, const void* k_pages,
-                                          const void* v_pages, const int32_t* block_tables,
-                                          uint32_t bt_stride, const int32_t* tiles,
-                                          uint32_t n_tiles, void* out, uint32_t n_heads,
-                                          uint32_t n_kv, void* stream) {
-  if (!qkv || !k_pages || !v_pages || !block_tables || !tiles || !out || n_kv == 0 ||
-      n_heads % n_kv) {
-    set_error("llmlb_op_prefill_attention: bad argument");
-    return LLMLB_E_INVALID_ARG;
-  }
-  if (n_tiles == 0) return LLMLB_OK;
-  constexpr size_t smem = (kPfRows + 4 * kPageTokens) * kHeadDim * 2;  // 80 KiB
-  static bool configured = false;
-  if (!configured) {
-    LLMLB_CUDA_CHECK(cudaFuncSetAttribute(prefill_attention_kernel,
-                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    configured = true;
-  }
-  dim3 grid(n_tiles, n_heads);
-  prefill_attention_kernel<<<grid, kPfThreads, smem, (cudaStream_t)stream>>>(
-      (const __nv_bfloat16*)qkv, (const __nv_bfloat16*)k_pages, (const __nv_bfloat16*)v_pages,
-      block_tables, bt_stride, (const int4*)tiles, (__nv_bfloat16*)out, n_heads, n_kv);
-  LLMLB_LAUNCH_CHECK();
-  return LLMLB_OK;
 }
 
 extern "C" size_t llmlb_op_decode_attention_ws(uint32_t, uint32_t, uint32_t) {
@@ -917,7 +709,7 @@ int decode_attention_launch(const void* qkv, void* k_pages, void* v_pages, const
   attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = (pdl && !(g_dbg_no_pdl & 8u)) ? 2 : 1;
+  cfg.numAttrs = pdl ? 2 : 1;
   LLMLB_CUDA_CHECK(cudaLaunchKernelEx(
       &cfg, decode_attention_kernel, (const __nv_bfloat16*)qkv, (__nv_bfloat16*)k_pages,
       (__nv_bfloat16*)v_pages, block_tables, bt_stride, bt_rows, seq_lens,

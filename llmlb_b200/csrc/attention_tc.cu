@@ -317,7 +317,7 @@ int prefill_attention_tc_launch(const CUtensorMap& mq, const CUtensorMap& mk, co
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = (pdl && !(g_dbg_no_pdl & 16u)) ? 1 : 0;
+  cfg.numAttrs = pdl ? 1 : 0;
   LLMLB_CUDA_CHECK(cudaLaunchKernelEx(&cfg, prefill_attention_kernel_tc, mq, mk, mv, layer, block_tables, bt_stride,
                                       (const int4*)tiles, (__nv_bfloat16*)out, n_heads, n_kv, pdl ? 1u : 0u));
   LLMLB_LAUNCH_CHECK();

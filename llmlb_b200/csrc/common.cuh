@@ -9,10 +9,6 @@
 
 namespace llmlb {
 
-// diagnostics: set once by llmlb_engine_create from LLMLB_DEBUG_NO_PDL (every launch then fully serialises behind its predecessor)
-extern unsigned int g_dbg_no_pdl;   // bit mask: 1 plain GEMV, 2 tp consumer GEMV, 4 tp push GEMV, 8 decode attention, 16 everything else
-
-
 constexpr int kHeadDim = 128;        // Llama-3 head width (the only one the kernels accept)
 constexpr int kPageTokens = 64;      // tokens per KV page
 constexpr int kNumSMs = 148;         // B200

@@ -60,9 +60,9 @@ void tc2_set_trace(const TraceBuf& tb);
 // tensor parallel (tp_common.cuh): fused GEMV consumer / producer of protocol A, pull kernels
 int gemv_tp_consume(const TpCtx& ctx, uint32_t coll_in, const void* w, const float* x_in, float* x_out,
                     const void* gain, float eps, void* out, uint32_t n_tokens, uint32_t n_out, uint32_t k,
-                    uint32_t epi, uint32_t out_stride, bool ll, bool gather, cudaStream_t st);
+                    uint32_t epi, uint32_t out_stride, cudaStream_t st);
 int gemv_tp_push(const TpCtx& ctx, uint32_t coll_out, const void* w, const void* x_bf16, uint32_t n_tokens,
-                 uint32_t n_out, uint32_t k, bool ll, cudaStream_t st);
+                 uint32_t n_out, uint32_t k, cudaStream_t st);
 int ar_allreduce_add(const TpCtx& P, uint64_t off, float* x, uint64_t n, cudaStream_t st);
 int ar_allgather_cols(const TpCtx& P, uint64_t off, float* out, uint32_t rows, uint32_t cols_local, cudaStream_t st);
 constexpr uint32_t kTpMaxSplit = 4;   // K-split parts a push-RS GEMM may use (slot capacity)
@@ -79,7 +79,6 @@ int rope_append_launch(void* qkv, const int32_t* positions, const int32_t* page_
 static thread_local std::string g_err;
 void set_error(const std::string& s) { g_err = s; }
 std::atomic<uint64_t> g_kernel_launches{0};
-unsigned int g_dbg_no_pdl = 0;
 
 #define RC(expr)                 \
   do {                           \
@@ -365,7 +364,7 @@ struct llmlb_engine {
   void* attn_ws = nullptr;
   CUtensorMap m_y[5]{}, m_attn[5]{}, m_h[5]{};  // box rows 16,32,64,128,256
   CUtensorMap m_attn_q{}, m_kpool{}, m_vpool{};  // tcgen05 prefill attention: q rows of qkv, the K / V pools (5-D)
-  uint32_t pf_tile = 128;                         // q rows per prefill-attention tile (64 for the mma.sync baseline)
+  static constexpr uint32_t kPfTile = 128;        // q rows per prefill-attention tile (UMMA M of attention_tc.cu)
 
   // per-step metadata (device) + pinned staging ring
   int32_t *d_ids = nullptr, *d_pos = nullptr, *d_page_of_tok = nullptr, *d_tiles = nullptr,
@@ -387,9 +386,6 @@ struct llmlb_engine {
   uint64_t logits_slot_off = 0, pull_slot_off = 0, pull_slot_bytes = 0;
   bool tp_ready = false;
   uint32_t tp_coll = 0;              // collectives issued so far in the current forward pass
-  bool tp_ll = true;                 // protocol A variant: {value, epoch} pairs (default) or values + end-of-grid flags
-  bool tp_gather = false;            // protocol A consumer: owner CTAs fold + in-GPU gather (tp_proto bit 1) instead of every CTA folding
-  bool dbg_no_ksplit = false, dbg_no_agwait = false, dbg_no_rsll = false, dbg_no_wave_tail = false;
   float* xb = nullptr;               // second residual buffer (protocol A ping-pong)
   float* tp_stage = nullptr;         // [4][hidden] fp32: partial rows of projections the fused GEMV does not take
   __nv_bfloat16* ylast = nullptr;    // [max_seqs][hidden] normalised rows that need logits (protocol B)
@@ -523,8 +519,8 @@ int llmlb_engine::init() {
   }
   if (!(tp == 1 || tp == 2 || tp == 4 || tp == 8) || rank >= tp) { set_error("bad tp_size/tp_rank"); return LLMLB_E_INVALID_ARG; }
   if (cfg.gemm_impl != 0) { set_error("gemm_impl: only 0 (tcgen05 tiles) is built into the library"); return LLMLB_E_INVALID_ARG; }
-  if (cfg.tp_proto > 3) { set_error("tp_proto: bit 0 = flags instead of value+epoch pairs, bit 1 = owner-fold + gather consumer"); return LLMLB_E_INVALID_ARG; }
-  if (cfg.attn_impl > 1) { set_error("attn_impl: 0 (tcgen05) or 1 (mma.sync baseline)"); return LLMLB_E_INVALID_ARG; }
+  if (cfg.attn_impl != 0) { set_error("attn_impl: only 0 (tcgen05 prefill attention) is built into the library"); return LLMLB_E_INVALID_ARG; }
+  if (cfg.tp_proto != 0) { set_error("tp_proto: only 0 ({value, epoch} pairs, every CTA folds) is built into the library"); return LLMLB_E_INVALID_ARG; }
   if (M.n_kv_heads == 0 || M.n_heads % M.n_kv_heads || M.n_kv_heads % tp || M.ffn % tp || M.vocab % tp ||
       ((M.n_heads / M.n_kv_heads) % 4) || M.hidden % 8 || (M.ffn / tp) % 8 || (M.vocab / tp) % 4 ||
       M.n_layers == 0 || M.vocab == 0) {
@@ -602,17 +598,6 @@ int llmlb_engine::alloc_all() {
   layer_pool_elems = size_t(n_pages) * nkv_l * kPageTokens * kHeadDim;
   RC(dmalloc(&k_pool, layer_pool_elems * M.n_layers));
   RC(dmalloc(&v_pool, layer_pool_elems * M.n_layers));
-  pf_tile = cfg.attn_impl == 0 ? 128 : 64;
-  tp_ll = (cfg.tp_proto & 1) == 0;
-  tp_gather = (cfg.tp_proto & 2) != 0;
-  // diagnostics, resolved once here (never read on the launch path)
-  g_dbg_no_pdl = getenv("LLMLB_DEBUG_NO_PDL") ? (unsigned int)atoi(getenv("LLMLB_DEBUG_NO_PDL")) : 0u;
-  dbg_no_ksplit = getenv("LLMLB_DEBUG_NO_KSPLIT") != nullptr;
-  dbg_no_rsll = getenv("LLMLB_DEBUG_NO_RSLL") != nullptr;
-  // measured (round 2, 512-token prefill): 66.1 k tok/s with the tail launch, 66.6 k without — the tail launch serialises
-  // behind the whole waves and pays its own ramp, so it stays opt-in (LLMLB_WAVE_TAIL=1)
-  dbg_no_wave_tail = getenv("LLMLB_WAVE_TAIL") == nullptr;
-  dbg_no_agwait = getenv("LLMLB_DEBUG_NO_AGWAIT") != nullptr;
   RC(make_tmap_attn_kv(&m_kpool, k_pool, M.n_layers, n_pages, nkv_l));
   RC(make_tmap_attn_kv(&m_vpool, v_pool, M.n_layers, n_pages, nkv_l));
   RC(dmalloc(&rope, size_t(cfg.max_ctx) * 64 * 2));
@@ -623,7 +608,7 @@ int llmlb_engine::alloc_all() {
   RC(dmalloc(&sk_ws, kSkWsBytes / 4, false));
   RC(dmalloc(&sk_cnt, kSkCounters));
   if (tp > 1) {
-    // the exchange region (tp_common.cuh): [pull barrier flags | TpFlags | slot 0 | slot 1 | logits | y]
+    // the exchange region (tp_common.cuh): [pull barrier flags | TpFlags | slots | pair slots | rs-pair slots | logits | y]
     const size_t al = 1024;
     auto up = [&](size_t v) { return (v + al - 1) & ~(al - 1); };
     const size_t slot = up(std::max(size_t(kTpMaxSplit) * (t_cap + kTpMaxRanks) * H * 4, size_t(kTpMaxRanks) * kTpSmallRows * H * 4));
@@ -639,9 +624,6 @@ int llmlb_engine::alloc_all() {
     const size_t rsslot = up(size_t(kTpMaxSplit) * (kTpLLTokens + kTpMaxRanks) * H * 4);   // parts x rows-per-owner <= split x (T + N)
     tpc.rsll_off[0] = off; off += rsslot;
     tpc.rsll_off[1] = off; off += rsslot;
-    const size_t gslot = up(size_t(kTpSmallRows) * H * 8);   // the consumer grid's own all-gather of the folded residual
-    tpc.gather_off[0] = off; off += gslot;
-    tpc.gather_off[1] = off; off += gslot;
     logits_slot_off = off; off += lslot;
     tpc.y_off = off; off += up(size_t(t_cap) * H * 2);
     xchg_bytes = off;
@@ -749,25 +731,9 @@ __global__ void gather_rows_bf16_kernel(const __nv_bfloat16* __restrict__ src, c
 int llmlb_engine::proj(const CUtensorMap& mw, const void*, const void*, const CUtensorMap* mx, void* out, uint32_t T,
                        uint32_t n_out, uint32_t k, uint32_t epi, uint32_t out_stride, int wait_coll) {
   TpPushRS tpp{};
-  if (!dbg_no_ksplit) { tpp.sk_ws = sk_ws; tpp.sk_cnt = sk_cnt; }   // narrow projections K-split inside the kernel
-  if (wait_coll >= 0 && !dbg_no_agwait) {   // tensor parallel: the activation operand is y of that collective (its all-gather flags gate the loads)
+  tpp.sk_ws = sk_ws; tpp.sk_cnt = sk_cnt;   // narrow projections K-split inside the kernel
+  if (wait_coll >= 0) {   // tensor parallel: the activation operand is y of that collective (its all-gather flags gate the loads)
     tpp.ctx = tpc; tpp.wait_coll_plus1 = uint32_t(wait_coll) + 1;
-  }
-  // A projection whose CTA-pair tiles fill whole waves plus a short ragged one (gate/up at 512 tokens: 224 tiles on
-  // 74 pairs = 3.03 waves, run as 4): the rows of the ragged wave go to a second launch of 128-row tiles with the
-  // in-kernel K-split (all SMs, a fraction of a tile time) and the pair kernel runs exact waves.
-  const bool store_epi = epi == LLMLB_EPI_STORE_BF16 || epi == LLMLB_EPI_SILU_MUL || epi == LLMLB_EPI_STORE_F32;
-  if (store_epi && T > 128 && n_out % 256 == 0 && tpp.sk_ws && !dbg_no_wave_tail) {
-    const uint32_t t_tiles = ceil_div(T, 256u), m_pairs = n_out / 256, pairs = uint32_t(kNumSMs / 2);
-    const uint32_t pair_tiles = m_pairs * t_tiles, waves = pair_tiles / pairs, rem = pair_tiles % pairs;
-    if (waves >= 2 && rem > 0 && rem % t_tiles == 0 && rem / t_tiles <= 2) {
-      const uint32_t rem_m = rem / t_tiles;
-      TpPushRS main = tpp, tail = tpp;
-      main.row0 = 0; main.n_rows = (m_pairs - rem_m) * 256;
-      tail.row0 = main.n_rows; tail.n_rows = rem_m * 256;
-      RC(gemm_tc_launch(mw, mx[bn_index(tc_pick_bn(T))], out, T, n_out, k, epi, out_stride, st, &mx[bn_index(128)], nullptr, &main));
-      return gemm_tc_launch(mw, mx[bn_index(tc_pick_bn(T))], out, T, n_out, k, epi, out_stride, st, &mx[bn_index(128)], nullptr, &tail);
-    }
   }
   return gemm_tc_launch(mw, mx[bn_index(tc_pick_bn(T))], out, T, n_out, k, epi, out_stride, st, &mx[bn_index(128)], nullptr, &tpp);
 }
@@ -779,11 +745,8 @@ int llmlb_engine::attention_block(uint32_t l, uint32_t T, bool decode, uint32_t 
                                    attn, nq_l, nkv_l, rope, decode_splits(nb), pdl, st);
   // both kernels are programmatic dependents: their set-up overlaps the tail of the kernel before
   RC(rope_append_launch(qkv, d_pos, d_page_of_tok, rope, kpool(l), vpool(l), T, nq_l, nkv_l, true, st));
-  if (cfg.attn_impl == 0)
-    return prefill_attention_tc_launch(m_attn_q, m_kpool, m_vpool, l, d_block_tables, pages_per_seq, d_tiles, n_tiles, attn,
-                                       nq_l, nkv_l, true, st);
-  return llmlb_op_prefill_attention(qkv, kpool(l), vpool(l), d_block_tables, pages_per_seq, d_tiles, n_tiles, attn,
-                                    nq_l, nkv_l, st);
+  return prefill_attention_tc_launch(m_attn_q, m_kpool, m_vpool, l, d_block_tables, pages_per_seq, d_tiles, n_tiles, attn,
+                                     nq_l, nkv_l, true, st);
 }
 
 // Runs the layer stack over T rows already embedded in x.  decode: rows are one new token per
@@ -849,9 +812,9 @@ int llmlb_engine::forward_small_tp(uint32_t T, bool decode, uint32_t nb, uint32_
   int pending = -1;   // collective pushed but not yet folded into `cur`
   auto consume = [&](const void* w, const __nv_bfloat16* gain, void* out, uint32_t n_out, uint32_t epi, uint32_t out_stride) -> int {
     if (pending >= 0) {
-      int rc = gemv_tp_consume(tpc, uint32_t(pending), w, cur, oth, gain, M.rms_eps, out, T, n_out, H, epi, out_stride, tp_ll, tp_gather, st);
+      int rc = gemv_tp_consume(tpc, uint32_t(pending), w, cur, oth, gain, M.rms_eps, out, T, n_out, H, epi, out_stride, st);
       if (rc == LLMLB_E_UNSUPPORTED) {   // odd shape: fold with its own kernel, then the plain projection
-        RC(tp_fold_rows(tpc, uint32_t(pending), cur, oth, T, H, tp_ll, st));
+        RC(tp_fold_rows(tpc, uint32_t(pending), cur, oth, T, H, st));
         rc = gemv_decode(w, oth, gain, M.rms_eps, out, T, n_out, H, epi, out_stride, st);
       }
       RC(rc);
@@ -863,10 +826,10 @@ int llmlb_engine::forward_small_tp(uint32_t T, bool decode, uint32_t nb, uint32_
   };
   auto push = [&](const void* w, const void* xin_bf16, uint32_t k) -> int {
     const uint32_t c = tp_coll++;
-    int rc = gemv_tp_push(tpc, c, w, xin_bf16, T, H, k, tp_ll, st);
+    int rc = gemv_tp_push(tpc, c, w, xin_bf16, T, H, k, st);
     if (rc == LLMLB_E_UNSUPPORTED) {
       RC(llmlb_op_gemv(w, xin_bf16, nullptr, M.rms_eps, tp_stage, T, H, k, LLMLB_EPI_STORE_F32, H, st));
-      rc = tp_push_rows(tpc, c, tp_stage, T, H, tp_ll, st);
+      rc = tp_push_rows(tpc, c, tp_stage, T, H, st);
     }
     RC(rc);
     pending = int(c);
@@ -887,7 +850,7 @@ int llmlb_engine::forward_small_tp(uint32_t T, bool decode, uint32_t nb, uint32_
 
 int llmlb_engine::finish_small_tp(FwdState* fs, uint32_t T) {
   if (!fs->pending) return LLMLB_OK;
-  RC(tp_fold_rows(tpc, fs->pending_coll, fs->xres, fs->xother, T, M.hidden, tp_ll, st));
+  RC(tp_fold_rows(tpc, fs->pending_coll, fs->xres, fs->xother, T, M.hidden, st));
   std::swap(fs->xres, fs->xother);
   fs->pending = false;
   return LLMLB_OK;
@@ -906,7 +869,7 @@ int llmlb_engine::forward_big_tp(uint32_t T, bool decode, uint32_t nb, uint32_t 
     tpp.ctx = tpc; tpp.coll = tp_coll++; tpp.rpr = rpr;
     *coll = int(tpp.coll);
     uint32_t n_parts = 1;
-    const bool ll = T <= kTpLLTokens && !dbg_no_rsll;   // narrow steps: {value, epoch} words, no flag round
+    const bool ll = T <= kTpLLTokens;   // narrow steps: {value, epoch} words, no flag round
     RC(gemm_tc_launch(mw, mx[bn_index(tc_pick_bn(T))], nullptr, T, H, k, ll ? kEpiPushRSLL : kEpiPushRS, H, st, &mx[bn_index(128)], &n_parts,
                       &tpp, kTpMaxSplit));
     return tp_reduce_norm(tpc, tpp.coll, x, next_gain, T, H, M.rms_eps, n_parts, last, ll, st);
@@ -955,7 +918,7 @@ int llmlb_engine::logits_from_y(const __nv_bfloat16* src, const CUtensorMap* map
 // protocol A, decode: the lm_head GEMV's prologue consumes the last down projection's collective
 int llmlb_engine::logits_tp_consume(FwdState* fs, uint32_t R) {
   int rc = gemv_tp_consume(tpc, fs->pending_coll, lm_head, fs->xres, fs->xother, final_norm, M.rms_eps, logits_dst(), R,
-                           vocab_l, M.hidden, LLMLB_EPI_STORE_F32, vocab_l, tp_ll, tp_gather, st);
+                           vocab_l, M.hidden, LLMLB_EPI_STORE_F32, vocab_l, st);
   if (rc == LLMLB_E_UNSUPPORTED) {
     RC(finish_small_tp(fs, R));
     return logits_from_x(fs->xres, R);
@@ -1084,9 +1047,9 @@ int llmlb_engine::run_prefill(const std::vector<ReqPtr>& reqs, const std::vector
       s_pos[row + j] = int32_t(pos);
       s_page[row + j] = r.pages[pos / kPageTokens];
     }
-    for (uint32_t j = 0; j < take[i]; j += pf_tile) {
+    for (uint32_t j = 0; j < take[i]; j += kPfTile) {
       s_tiles[n_tiles * 4 + 0] = int32_t(row + j);
-      s_tiles[n_tiles * 4 + 1] = int32_t(std::min<uint32_t>(pf_tile, take[i] - j));
+      s_tiles[n_tiles * 4 + 1] = int32_t(std::min<uint32_t>(kPfTile, take[i] - j));
       s_tiles[n_tiles * 4 + 2] = int32_t(p0 + j);
       s_tiles[n_tiles * 4 + 3] = r.slot;
       ++n_tiles;
@@ -1909,7 +1872,7 @@ extern "C" int llmlb_debug_prefill_logits(llmlb_engine* e, const int32_t* prompt
   const int slot = e->debug_slot;
   std::vector<int32_t> pos(n), page(n), tiles;
   for (uint32_t i = 0; i < n; ++i) { pos[i] = int32_t(i); page[i] = e->debug_pages[i / kPageTokens]; }
-  for (uint32_t j = 0; j < n; j += e->pf_tile) { tiles.push_back(int32_t(j)); tiles.push_back(int32_t(std::min<uint32_t>(e->pf_tile, n - j))); tiles.push_back(int32_t(j)); tiles.push_back(slot); }
+  for (uint32_t j = 0; j < n; j += llmlb_engine::kPfTile) { tiles.push_back(int32_t(j)); tiles.push_back(int32_t(std::min<uint32_t>(llmlb_engine::kPfTile, n - j))); tiles.push_back(int32_t(j)); tiles.push_back(slot); }
   LLMLB_CUDA_CHECK(cudaMemcpy(e->d_block_tables + size_t(slot) * e->pages_per_seq, e->debug_pages.data(), e->debug_pages.size() * 4, cudaMemcpyHostToDevice));
   LLMLB_CUDA_CHECK(cudaMemcpy(e->d_ids, prompt, n * 4, cudaMemcpyHostToDevice));
   LLMLB_CUDA_CHECK(cudaMemcpy(e->d_pos, pos.data(), n * 4, cudaMemcpyHostToDevice));

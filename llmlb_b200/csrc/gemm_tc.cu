@@ -55,7 +55,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant
   const uint32_t k_blocks_total = (K + kBK - 1) / kBK;
   const uint32_t k_per_split = (k_blocks_total + split_k - 1) / split_k;
   const uint32_t n_tiles = m_tiles * t_tiles * split_k;
-  const uint32_t m_tile0 = tp.row0 / kBM;
 
   if (warp == 0 && lane == 0) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(&tmap_w) : "memory");
@@ -96,7 +95,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant
     tt = tile % t_tiles;
     uint32_t r = tile / t_tiles;
     ks = r % split_k;
-    mt = r / split_k + m_tile0;
+    mt = r / split_k;
   };
 
   if (warp == 0) {
@@ -217,7 +216,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant
           // group (sum over the parts in part order: deterministic), so the reduction itself is spread
           // over the CTAs that did the products.  All CTAs of the grid are co-resident (one tile per CTA,
           // grid <= SM count) and nobody waits before it has parked its own part.
-          const uint32_t otile = (mt - m_tile0) * t_tiles + tt;
+          const uint32_t otile = mt * t_tiles + tt;
           float* wtile = tp.sk_ws + size_t(otile) * split_k * (BN * kBM);
           float* wmine = wtile + size_t(ks) * (BN * kBM);
 #pragma unroll 1
@@ -477,8 +476,7 @@ static int launch_tc(const CUtensorMap& tw, const CUtensorMap& tx, void* out, ui
   }
   TpPushRS tp{};
   if (tpp) tp = *tpp;
-  const uint32_t rows = tp.n_rows ? tp.n_rows : n_out;
-  uint32_t m_tiles = (rows + kBM - 1) / kBM;
+  uint32_t m_tiles = (n_out + kBM - 1) / kBM;
   uint32_t t_tiles = (n_tokens + BN - 1) / BN;
   uint32_t tiles = m_tiles * t_tiles * split_k;
   uint32_t grid = tiles < (uint32_t)kNumSMs ? tiles : (uint32_t)kNumSMs;
@@ -497,7 +495,7 @@ static int launch_tc(const CUtensorMap& tw, const CUtensorMap& tx, void* out, ui
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = (g_dbg_no_pdl & 16u) ? 0 : 1;
+    cfg.numAttrs = 1;
     LLMLB_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kern, tw, tx, out, n_tokens, n_out, k, out_stride, m_tiles, t_tiles, split_k, 1u, tp));
   }
   LLMLB_LAUNCH_CHECK();
@@ -535,8 +533,7 @@ static int dispatch_tc_epi(uint32_t epi, const CUtensorMap& tw, const CUtensorMa
 uint32_t tc_store_split(uint32_t n_tokens, uint32_t n_out, uint32_t k, const TpPushRS* tpp) {
   if (!tpp || !tpp->sk_ws || !tpp->sk_cnt) return 1;
   const uint32_t bn = tc_pick_bn(n_tokens);
-  const uint32_t rows = tpp->n_rows ? tpp->n_rows : n_out;
-  const uint32_t tiles = ((rows + kBM - 1) / kBM) * ((n_tokens + bn - 1) / bn);
+  const uint32_t tiles = ((n_out + kBM - 1) / kBM) * ((n_tokens + bn - 1) / bn);
   const uint32_t kblocks = (k + kBK - 1) / kBK;
   if (tiles * 2 > (uint32_t)kNumSMs || tiles > kSkCounters) return 1;
   uint32_t s = (uint32_t)kNumSMs / tiles;
@@ -575,15 +572,14 @@ int gemm_tc_launch(const CUtensorMap& tw, const CUtensorMap& tx, void* out, uint
   // CTA pairs when there are enough 256 x 256 tiles to occupy most of the GPU; a narrow projection (tensor-
   // parallel shards: QKV at tp = 8 has 6 pair tiles) runs 128-row tiles with an in-kernel K-split instead
   const bool store_epi = epi == LLMLB_EPI_STORE_BF16 || epi == LLMLB_EPI_SILU_MUL || epi == LLMLB_EPI_STORE_F32;
-  const uint32_t rows_w = (tpp && tpp->n_rows) ? tpp->n_rows : n_out;
-  const uint32_t pair_ctas = 2 * ((rows_w + 255) / 256) * ((n_tokens + 255) / 256);
+  const uint32_t pair_ctas = 2 * ((n_out + 255) / 256) * ((n_tokens + 255) / 256);
   const bool narrow = store_epi && pair_ctas < 96 && tc_store_split(n_tokens, n_out, k, tpp) > 1;
   if (tx_half && bn == 256 && n_out >= 256 && !narrow)
     return gemm_tc2_launch(tw, *tx_half, out, n_tokens, n_out, k, epi, out_stride, st, n_parts, tpp, max_split);
   // split K for the residual epilogues when the tile count cannot fill the GPU
   uint32_t split_k = 1;
   if (epi == LLMLB_EPI_RESID_F32 || epi == (uint32_t)kEpiPartialF32 || epi == (uint32_t)kEpiPushRS || epi == (uint32_t)kEpiPushRSLL) {
-    uint32_t tiles = ((rows_w + kBM - 1) / kBM) * ((n_tokens + bn - 1) / bn);
+    uint32_t tiles = ((n_out + kBM - 1) / kBM) * ((n_tokens + bn - 1) / bn);
     uint32_t kblocks = (k + kBK - 1) / kBK;
     while (tiles * split_k * 2 <= (uint32_t)kNumSMs && kblocks / (split_k * 2) >= 8 && split_k * 2 <= max_split) split_k *= 2;
   } else {

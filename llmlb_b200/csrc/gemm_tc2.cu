@@ -77,7 +77,6 @@ __global__ void __launch_bounds__(kTcThreads, 1)
 gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant__ CUtensorMap tmap_x,
                 void* __restrict__ out, uint32_t n_tokens, uint32_t n_out, uint32_t K, uint32_t out_stride,
                 uint32_t m_tiles /*256-row slabs*/, uint32_t t_tiles, uint32_t split_k, const TpPushRS tp) {
-  const uint32_t m_tile0 = tp.row0 / 256;
   using Cfg = Tc2Cfg<BN>;
   const TraceBuf tb = d_trace_tc2;
   unsigned long long tr0 = 0, tr1 = 0;
@@ -138,7 +137,7 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constan
     tt = tile % t_tiles;
     uint32_t r = tile / t_tiles;
     ks = r % split_k;
-    mt = r / split_k + m_tile0;
+    mt = r / split_k;
   };
 
   if (warp == 0) {
@@ -279,8 +278,7 @@ static int launch_tc2(const CUtensorMap& tw, const CUtensorMap& tx_half, void* o
   }
   TpPushRS tp{};
   if (tpp) tp = *tpp;
-  const uint32_t rows = tp.n_rows ? tp.n_rows : n_out;
-  const uint32_t m_tiles = (rows + 255) / 256, t_tiles = (n_tokens + BN - 1) / BN;
+  const uint32_t m_tiles = (n_out + 255) / 256, t_tiles = (n_tokens + BN - 1) / BN;
   const uint32_t tiles = m_tiles * t_tiles * split_k;
   uint32_t pairs = tiles < (uint32_t)(kNumSMs / 2) ? tiles : (uint32_t)(kNumSMs / 2);
   cudaLaunchConfig_t cfg{};
@@ -296,7 +294,7 @@ static int launch_tc2(const CUtensorMap& tw, const CUtensorMap& tx_half, void* o
   attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = (g_dbg_no_pdl & 16u) ? 1 : 2;
+  cfg.numAttrs = 2;
   LLMLB_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kern, tw, tx_half, out, n_tokens, n_out, k, out_stride, m_tiles, t_tiles, split_k, tp));
   LLMLB_LAUNCH_CHECK();
   return LLMLB_OK;
@@ -308,7 +306,7 @@ int gemm_tc2_launch(const CUtensorMap& tw, const CUtensorMap& tx_half, void* out
                     const TpPushRS* tpp, uint32_t max_split) {
   uint32_t split_k = 1;
   if (epi == LLMLB_EPI_RESID_F32 || epi == (uint32_t)kEpiPartialF32 || epi == (uint32_t)kEpiPushRS) {
-    uint32_t tiles = (((tpp && tpp->n_rows ? tpp->n_rows : n_out) + 255) / 256) * ((n_tokens + 255) / 256);
+    uint32_t tiles = ((n_out + 255) / 256) * ((n_tokens + 255) / 256);
     uint32_t kblocks = (k + kBK - 1) / kBK;
     while (tiles * split_k * 2 <= (uint32_t)(kNumSMs / 2) && kblocks / (split_k * 2) >= 8 && split_k * 2 <= max_split) split_k *= 2;
   }

@@ -22,18 +22,17 @@
 namespace llmlb {
 
 // Tensor-parallel decode (protocol A of tp_common.cuh), fused into this kernel:
-//   TPM == 1  the RMSNorm prologue is the all-reduce's consumer: wait for the N push flags, fold the
-//             N partial rows of the slot into the replicated fp32 residual (rank order), keep the
-//             new residual in shared memory for the norm and write it to x_out (the other residual
-//             buffer: other CTAs of this grid still read x_in)
-//   TPM == 2  the epilogue is the producer: every finished output element is stored into the slot
-//             of EVERY rank, the last CTA of the grid raises the flags
+//   TPM == 1  the RMSNorm prologue is the all-reduce's consumer: every CTA folds the N partial rows
+//             of the slot into the replicated fp32 residual (rank order), spinning on the epoch of
+//             each {value, epoch} pair, keeps the new residual in shared memory for the norm and
+//             writes its share of it to x_out (the other residual buffer: other CTAs of this grid
+//             still read x_in)
+//   TPM == 2  the epilogue is the producer: every finished output element is stored with its epoch
+//             into the slot of EVERY rank (no flag, no end-of-grid signal)
 struct TpGemv {
   TpCtx ctx;
   uint32_t coll_in, coll_out;   // collective consumed by the prologue / produced by the epilogue
   float* x_out;                 // TPM == 1: residual after the fold
-  uint32_t ll;                  // 1: {value, epoch} pairs (no flags), 0: values + end-of-grid flags
-  uint32_t gather;              // TPM == 1: 1 = owner CTAs fold, the grid gathers the result through L2; 0 = every CTA folds
 };
 
 constexpr int kKsThreads = 512;
@@ -95,7 +94,7 @@ gemv_ks_kernel(const __nv_bfloat16* __restrict__ W, const void* xin /* predecess
   // ... and only now wait for the producer of x / out (weights above never depend on it)
   asm volatile("griddepcontrol.wait;" ::: "memory");
   if (tb.data && threadIdx.x == 0) tr1 = gtime_ns();
-  uint32_t ep_out = 0;   // TPM == 2, LL: the epoch every pushed value carries (step counter is final after the wait)
+  uint32_t ep_out = 0;   // TPM == 2: the epoch every pushed value carries (step counter is final after the wait)
   if constexpr (TPM == 2) ep_out = tp_epoch32(tp.ctx, tp.coll_out);
 
   // ---- prologue: this lane's slice of x in fp32 registers (RMSNorm fused) ----
@@ -109,84 +108,40 @@ gemv_ks_kernel(const __nv_bfloat16* __restrict__ W, const void* xin /* predecess
       const uint32_t slot = tp.coll_in & 1;
       TpFlags* mine = tp_flags(tp.ctx, tp.ctx.rank);
       const uint32_t ep32 = tp_epoch32(tp.ctx, tp.coll_in);
-      if (!tp.ll) {
-        tp_wait_flags(mine, mine->push_flag[slot], tp.ctx.size, tp_epoch(tp.ctx, tp.coll_in));
-        if (tb.data && threadIdx.x == 0) tr_flag = gtime_ns();
-      }
-      const uint8_t* slot_base = tp.ctx.base[tp.ctx.rank] + (tp.ll ? tp.ctx.ll_off[slot] : tp.ctx.slot_off[slot]);
-      uint4* gat = reinterpret_cast<uint4*>(tp.ctx.base[tp.ctx.rank] + tp.ctx.gather_off[slot]);
+      const uint8_t* slot_base = tp.ctx.base[tp.ctx.rank] + tp.ctx.ll_off[slot];
       // x_in[b][4i..4i+3] + the N pushed partials, summed in rank order (identical sums on every rank); the loads
       // of up to four sources are issued together
       auto fold_one = [&](int b, uint32_t i) -> float4 {
         float4 v = reinterpret_cast<const float4*>(xf + size_t(b) * K)[i];
         for (uint32_t r0 = 0; r0 < tp.ctx.size; r0 += 4) {
-          if (tp.ll) {
-            const uint4* pp[4];
-            uint4 pa[4], pb[4];
+          const uint4* pp[4];
+          uint4 pa[4], pb[4];
 #pragma unroll
-            for (int q = 0; q < 4; ++q)
-              if (r0 + q < tp.ctx.size) {
-                pp[q] = reinterpret_cast<const uint4*>(slot_base) + ((size_t(r0 + q) * kTpSmallRows + b) * K + 4 * size_t(i)) / 2;
-                pa[q] = ld_pairs(pp[q]); pb[q] = ld_pairs(pp[q] + 1);
-              }
+          for (int q = 0; q < 4; ++q)
+            if (r0 + q < tp.ctx.size) {
+              pp[q] = reinterpret_cast<const uint4*>(slot_base) + ((size_t(r0 + q) * kTpSmallRows + b) * K + 4 * size_t(i)) / 2;
+              pa[q] = ld_pairs(pp[q]); pb[q] = ld_pairs(pp[q] + 1);
+            }
 #pragma unroll
-            for (int q = 0; q < 4; ++q)
-              if (r0 + q < tp.ctx.size) {
-                const float4 a = tp_take_pairs(mine, pp[q], pa[q], pb[q], ep32);
-                v.x += a.x; v.y += a.y; v.z += a.z; v.w += a.w;
-              }
-          } else {
-            float4 a[4];
-#pragma unroll
-            for (int q = 0; q < 4; ++q)
-              if (r0 + q < tp.ctx.size)
-                a[q] = ld_pushed_f4(reinterpret_cast<const float4*>(slot_base) + (size_t(r0 + q) * kTpSmallRows + b) * (K / 4) + i);
-#pragma unroll
-            for (int q = 0; q < 4; ++q)
-              if (r0 + q < tp.ctx.size) { v.x += a[q].x; v.y += a[q].y; v.z += a[q].z; v.w += a[q].w; }
-          }
+          for (int q = 0; q < 4; ++q)
+            if (r0 + q < tp.ctx.size) {
+              const float4 a = tp_take_pairs(mine, pp[q], pa[q], pb[q], ep32);
+              v.x += a.x; v.y += a.y; v.z += a.z; v.w += a.w;
+            }
         }
         return v;
       };
-      if (tp.gather) {
-        // (1) OWNER FOLD.  float4 i of every row belongs to CTA i % gridDim.x: only that CTA reads the N pushed
-        // partials (every CTA folding the whole residual costs 148 x N x K x 8 B of L2 reads per launch: 39 MB at
-        // N = 8), writes the new residual and publishes it to the rest of the grid as {value, epoch} pairs.
-        for (uint32_t i = blockIdx.x + gridDim.x * threadIdx.x; i < K / 4; i += gridDim.x * kKsThreads) {
+      // every CTA folds the whole residual itself (one L2 hop after the push lands)
+      for (uint32_t i = threadIdx.x; i < K / 4; i += kKsThreads) {
 #pragma unroll
-          for (int b = 0; b < B; ++b) {
-            const float4 v = fold_one(b, i);
-            reinterpret_cast<float4*>(tp.x_out + size_t(b) * K)[i] = v;
-            uint4* g = gat + (size_t(b) * K + 4 * size_t(i)) / 2;
-            st_pairs_gpu(g, v.x, v.y, ep32);
-            st_pairs_gpu(g + 1, v.z, v.w, ep32);
-          }
-        }
-        // (2) GATHER.  Every CTA reads the whole folded residual back from L2 (K x 8 B per row), spinning on
-        // the epochs of pieces whose owner CTA is not through yet.  All CTAs of the grid are co-resident
-        // (grid <= SM count, one CTA per SM) and every owner publishes BEFORE it spins: no circular wait.
-        for (uint32_t i = threadIdx.x; i < K / 4; i += kKsThreads) {
-#pragma unroll
-          for (int b = 0; b < B; ++b) {
-            const uint4* g = gat + (size_t(b) * K + 4 * size_t(i)) / 2;
-            const float4 v = tp_take_pairs_gpu(mine, g, ld_pairs_gpu(g), ld_pairs_gpu(g + 1), ep32);
-            reinterpret_cast<float4*>(ks_dyn + size_t(b) * K)[i] = v;
-            ss[b] += v.x * v.x + v.y * v.y + v.z * v.z + v.w * v.w;
-          }
-        }
-      } else {
-        // every CTA folds the whole residual itself (one L2 hop after the push lands)
-        for (uint32_t i = threadIdx.x; i < K / 4; i += kKsThreads) {
-#pragma unroll
-          for (int b = 0; b < B; ++b) {
-            const float4 v = fold_one(b, i);
-            reinterpret_cast<float4*>(ks_dyn + size_t(b) * K)[i] = v;
-            if (i % gridDim.x == blockIdx.x) reinterpret_cast<float4*>(tp.x_out + size_t(b) * K)[i] = v;
-            ss[b] += v.x * v.x + v.y * v.y + v.z * v.z + v.w * v.w;
-          }
+        for (int b = 0; b < B; ++b) {
+          const float4 v = fold_one(b, i);
+          reinterpret_cast<float4*>(ks_dyn + size_t(b) * K)[i] = v;
+          if (i % gridDim.x == blockIdx.x) reinterpret_cast<float4*>(tp.x_out + size_t(b) * K)[i] = v;
+          ss[b] += v.x * v.x + v.y * v.y + v.z * v.z + v.w * v.w;
         }
       }
-      if (tp.ll && tb.data && threadIdx.x == 0) tr_flag = gtime_ns();
+      if (tb.data && threadIdx.x == 0) tr_flag = gtime_ns();
       xf = ks_dyn;   // generic pointer into shared memory: the slices below come from the fold
     } else {
     for (uint32_t i = threadIdx.x; i < K / 4; i += kKsThreads) {
@@ -303,13 +258,8 @@ gemv_ks_kernel(const __nv_bfloat16* __restrict__ W, const void* xin /* predecess
         if (lane < RB * B && row < rows_lim) {
           const size_t idx = (size_t(tp.ctx.rank) * kTpSmallRows + b) * out_stride + row;
           const uint32_t slot = tp.coll_out & 1;
-          if (tp.ll) {
-            for (uint32_t r = 0; r < tp.ctx.size; ++r)
-              st_peer_pair(reinterpret_cast<uint2*>(tp.ctx.base[r] + tp.ctx.ll_off[slot]) + idx, v, ep_out);
-          } else {
-            for (uint32_t r = 0; r < tp.ctx.size; ++r)
-              st_peer_f32(reinterpret_cast<float*>(tp.ctx.base[r] + tp.ctx.slot_off[slot]) + idx, v);
-          }
+          for (uint32_t r = 0; r < tp.ctx.size; ++r)
+            st_peer_pair(reinterpret_cast<uint2*>(tp.ctx.base[r] + tp.ctx.ll_off[slot]) + idx, v, ep_out);
         }
       } else if (lane < RB * B && row < rows_lim) {
         const size_t idx = size_t(b) * out_stride + row;
@@ -328,14 +278,9 @@ gemv_ks_kernel(const __nv_bfloat16* __restrict__ W, const void* xin /* predecess
   // and the next one launches (the boundary otherwise leaves HBM idle for ~2-3 us) ----
   for (uint32_t off = (blockIdx.x * kKsThreads + threadIdx.x) * 128u; off < pf_bytes; off += gridDim.x * kKsThreads * 128u)
     asm volatile("prefetch.global.L2 [%0];" ::"l"(pf_ptr + off));
-  if (TPM == 2 && !tp.ll) {
-    const uint32_t slot = tp.coll_out & 1;
-    tp_signal_when_grid_done(tp.ctx, &tp_flags(tp.ctx, tp.ctx.rank)->done[slot], gridDim.x, tp_epoch(tp.ctx, tp.coll_out),
-                             [&](TpFlags* f) { return &f->push_flag[slot][tp.ctx.rank]; });
-  }
   if (tb.data && threadIdx.x == 0) {
     trace_emit(tb, ((unsigned long long)TPM << 58) | ((unsigned long long)n_out << 32) | K, tr0, tr1, tr2, gtime_ns());
-    if (TPM == 1) trace_emit(tb, (5ull << 60) | ((unsigned long long)n_out << 32) | K, tr1, tr_flag, tr2, 0);   // dependency wait -> flags in -> fold + norm done
+    if (TPM == 1) trace_emit(tb, (5ull << 60) | ((unsigned long long)n_out << 32) | K, tr1, tr_flag, tr2, 0);   // dependency wait -> fold done -> norm done
   }
 }
 
@@ -376,7 +321,7 @@ static int ks_launch(const void* w, const void* x, const void* gain, float eps, 
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;  // programmatic dependent launch
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = (g_dbg_no_pdl & (TPM == 0 ? 1u : TPM == 1 ? 2u : 4u)) ? 0 : 1;
+  cfg.numAttrs = 1;
   TpGemv tpv{};
   if (tp) tpv = *tp;
   LLMLB_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kern, (const __nv_bfloat16*)w, x,
@@ -429,11 +374,11 @@ bool gemv_tp_shape_ok(uint32_t n_tokens, uint32_t k) {
 // consumer: x_out = x_in + sum of the pushed partials of collective coll_in; out = epi(W . RMSNorm(x_out))
 int gemv_tp_consume(const TpCtx& ctx, uint32_t coll_in, const void* w, const float* x_in, float* x_out,
                     const void* gain, float eps, void* out, uint32_t n_tokens, uint32_t n_out, uint32_t k,
-                    uint32_t epi, uint32_t out_stride, bool ll, bool gather, cudaStream_t st) {
+                    uint32_t epi, uint32_t out_stride, cudaStream_t st) {
   uint32_t tw = 0, cw = 0;
   if (n_tokens == 0 || n_tokens > 4 || !gain || !ks_pick(n_tokens, k, &tw, &cw)) return LLMLB_E_UNSUPPORTED;
   TpGemv tp{};
-  tp.ctx = ctx; tp.coll_in = coll_in; tp.x_out = x_out; tp.ll = ll ? 1u : 0u; tp.gather = gather ? 1u : 0u;
+  tp.ctx = ctx; tp.coll_in = coll_in; tp.x_out = x_out;
 #define KS_TC(BB, CC)                                                                                                          \
   switch (epi) {                                                                                                               \
     case LLMLB_EPI_STORE_BF16: return ks_launch<BB, LLMLB_EPI_STORE_BF16, true, CC, 1>(w, x_in, gain, eps, out, n_out, k, out_stride, tw, st, nullptr, 0, &tp); \
@@ -450,11 +395,11 @@ int gemv_tp_consume(const TpCtx& ctx, uint32_t coll_in, const void* w, const flo
 
 // producer: partial = W . x (bf16 x) pushed into slot[coll_out & 1][my rank] of every rank (n_out = hidden)
 int gemv_tp_push(const TpCtx& ctx, uint32_t coll_out, const void* w, const void* x_bf16, uint32_t n_tokens,
-                 uint32_t n_out, uint32_t k, bool ll, cudaStream_t st) {
+                 uint32_t n_out, uint32_t k, cudaStream_t st) {
   uint32_t tw = 0, cw = 0;
   if (n_tokens == 0 || n_tokens > 4 || !ks_pick(n_tokens, k, &tw, &cw)) return LLMLB_E_UNSUPPORTED;
   TpGemv tp{};
-  tp.ctx = ctx; tp.coll_out = coll_out; tp.ll = ll ? 1u : 0u;
+  tp.ctx = ctx; tp.coll_out = coll_out;
 #define KS_TP(BB, CC) return ks_launch<BB, LLMLB_EPI_STORE_F32, false, CC, 2>(w, x_bf16, nullptr, 0.f, nullptr, n_out, k, n_out, tw, st, nullptr, 0, &tp)
   if (n_tokens == 1) { if (cw == 1) KS_TP(1, 1); if (cw == 2) KS_TP(1, 2); KS_TP(1, 4); }
   if (n_tokens == 2) { if (cw == 1) KS_TP(2, 1); KS_TP(2, 2); }

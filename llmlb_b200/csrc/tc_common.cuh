@@ -29,9 +29,6 @@ struct TpPushRS {
   // one arrival counter per output tile in sk_cnt (zero between launches); nullptr = no K-split
   float* sk_ws;
   unsigned int* sk_cnt;
-  // row window of W this launch covers (a projection may be issued as whole waves of CTA-pair tiles plus a K-split
-  // tail launch for the rows of the ragged last wave): rows [row0, row0 + n_rows), n_rows == 0 = all rows
-  uint32_t row0, n_rows;
 };
 constexpr size_t kSkWsBytes = size_t(148) * 128 * 256 * 4;   // every CTA of a full grid parks one 128 x 256 fp32 tile
 constexpr uint32_t kSkCounters = 256;

@@ -2,33 +2,39 @@
 //
 // Every rank owns ONE CUDA-IPC-shared exchange region, mapped into all peers:
 //
-//   [ ArSignals | TpFlags | slot 0 | slot 1 | logits slot | y (bf16 activations, t_cap x hidden) ]
+//   [ ArSignals | TpFlags | slot 0 | slot 1 | pair slot 0 | pair slot 1 | rs-pair slot 0 | rs-pair slot 1 |
+//     logits slot | y (bf16 activations, t_cap x hidden) ]
 //
-// Two protocols, both PUSH based (a producer stores into its peers' memory, then raises a flag;
-// nobody ever reads remote memory, so a consumer only pays local L2 latency after the flag):
+// Two protocols, both PUSH based (a producer stores into its peers' memory; nobody ever reads
+// remote memory, so a consumer only pays local L2 latency once the data has landed):
 //
-//  A  "one-shot push", T <= 4 rows (decode).  The O / down projection GEMV writes its fp32 partial
-//     row into slot[coll & 1][src = my rank] of EVERY rank and the last CTA of the grid raises
-//     push_flag[slot][my rank] on every rank.  The CONSUMER is the next projection's RMSNorm
-//     prologue (gate/up, next QKV, lm_head): it waits for the N flags, folds the N partials into
-//     the replicated fp32 residual in rank order (bit-identical on every rank) and normalises —
-//     no separate all-reduce kernel, no barrier round trip.
+//  A  "one-shot push", T <= 4 rows (decode).  The O / down projection GEMV stores every fp32
+//     partial value together with the collective's 32-bit epoch as ONE 8-byte {value, epoch} pair
+//     into pair slot[coll & 1][src = my rank] of EVERY rank.  8-byte stores are single-copy atomic,
+//     so a consumer that reads a pair carrying its epoch has the value: no fence, no ticket, no
+//     flag.  The CONSUMER is the next projection's RMSNorm prologue (gate/up, next QKV, lm_head):
+//     every CTA spins on the epochs of the pairs, folds the N partials into the replicated fp32
+//     residual in rank order (bit-identical on every rank) and normalises — no separate all-reduce
+//     kernel, no barrier round trip.
 //
 //  B  "reduce-scatter + all-gather", T > 4 rows (prefill, batched decode).  Token rows are dealt
 //     to owner ranks in chunks of rpr = ceil(T / N).  The O / down projection GEMM's epilogue
-//     stores each fp32 partial tile row straight into the OWNER's slot[.][src][row] (reduce-
-//     scatter by address), last CTA raises push_flag on every rank.  tp_reduce_norm_kernel, one
-//     CTA per owned row: waits for the N flags, x[row] += sum of the N partials (the residual is
-//     row-sharded: only the owner keeps it), RMSNorm, and stores the bf16 row into the `y`
-//     buffer of EVERY rank (all-gather by address, bf16 on the wire); the last CTA raises ag_flag
-//     everywhere and CTA 0 does not exit before all N ag_flags arrived, so the next GEMM's TMA
-//     loads of y are ordered by the kernel boundary.
+//     stores each partial tile row, as bf16, straight into the OWNER's slot (reduce-scatter by
+//     address).  Wide steps (T > kTpLLTokens) write slot[.][part][row] and the last CTA raises
+//     push_flag on every rank; narrow steps write {bf16 x 2, epoch} words into the rs-pair slot and
+//     raise no flag.  tp_reduce_norm_kernel, one CTA per owned row: waits for the N flags (or the
+//     words' epochs), x[row] += sum of the partials (the residual is row-sharded: only the owner
+//     keeps it), RMSNorm, and stores the bf16 row into the `y` buffer of EVERY rank (all-gather by
+//     address); the last CTA raises ag_flag everywhere.  The GEMM that consumes y waits for the
+//     N ag_flags in its TMA producer (tp_wait_ag_single); for any other consumer the reduce kernel's
+//     CTA 0 does not exit before all N ag_flags arrived, so the kernel boundary orders the loads.
 //
-// Flags hold epochs, never reset: epoch = (step << 12) | (collective index within the step + 1),
+// Flags hold 64-bit epochs, never reset: epoch = (step << 12) | (collective index within the step + 1),
 // `step` is bumped by tp_step_begin_kernel at the start of every forward pass, identically on all
-// ranks (they launch identical steps).  64-bit, so no wrap.  Slots alternate per collective; a rank
-// can never be more than one collective ahead of a peer (it needs the peer's push to finish its
-// own consumer), so two slots suffice.
+// ranks (they launch identical steps).  Pairs carry the 32-bit form (tp_epoch32).  Slots alternate
+// per collective; a rank can never be more than one collective ahead of a peer (it needs the peer's
+// push to finish its own consumer), so two slots suffice.  Slot 0 also serves the standalone pull
+// all-reduce (llmlb_op_allreduce).
 #pragma once
 #include <stdint.h>
 
@@ -55,13 +61,11 @@ struct TpCtx {                      // kernel parameter, by value
   uint8_t* base[kTpMaxRanks];       // exchange region of every rank (peer-mapped)
   uint32_t rank, size;
   uint64_t flags_off;               // TpFlags
-  uint64_t slot_off[kTpSlots];      // fp32 partial slots
-  uint64_t ll_off[kTpSlots];        // {value, epoch} pair slots of the LL variant (never written by anything else,
-                                    // so a stale word can only be an older epoch)
+  uint64_t slot_off[kTpSlots];      // protocol B, wide steps: bf16 partials of the reduce-scatter [part][row][hidden]
+  uint64_t ll_off[kTpSlots];        // protocol A: {value, epoch} pairs [src][kTpSmallRows][hidden] (never written by
+                                    // anything else, so a stale word can only be an older epoch)
   uint64_t rsll_off[kTpSlots];      // protocol B, narrow steps: {bf16 x 2, epoch} words of the reduce-scatter
                                     // [part][row of the owner][hidden / 2] (never written by anything else)
-  uint64_t gather_off[kTpSlots];    // protocol A consumer: the folded residual as {value, epoch} pairs, written by the
-                                    // owner CTAs of THIS rank's consumer grid and read back by all of its CTAs
   uint64_t y_off;                   // bf16 [t_cap, hidden] normalised activations
   uint64_t slot_bytes;
 };
@@ -89,9 +93,6 @@ __device__ __forceinline__ float4 ld_pushed_f4(const float4* p) {
                : "memory");
   return v;
 }
-__device__ __forceinline__ void st_peer_f32(float* p, float v) {
-  asm volatile("st.relaxed.sys.global.f32 [%0], %1;" ::"l"(p), "f"(v) : "memory");
-}
 __device__ __forceinline__ void st_peer_bf16(__nv_bfloat16* p, float v) {   // reduce-scatter partials travel as bf16
   const unsigned short b = __bfloat16_as_ushort(__float2bfloat16_rn(v));
   asm volatile("st.relaxed.sys.global.u16 [%0], %1;" ::"l"(p), "h"(b) : "memory");
@@ -104,25 +105,15 @@ __device__ __forceinline__ uint2 ld_pushed_u2(const uint2* p) {
 __device__ __forceinline__ void st_peer_u2(void* p, uint2 v) {
   asm volatile("st.relaxed.sys.global.v2.u32 [%0], {%1,%2};" ::"l"(p), "r"(v.x), "r"(v.y) : "memory");
 }
-// ---- "LL" variant of protocol A: every pushed value travels with its epoch in ONE 8-byte store
-// {value bits, epoch32}.  8-byte stores are single-copy atomic, so a consumer that reads the pair and
-// finds its epoch has the value: no fence, no ticket, no flag, no last-CTA — the push is visible one
-// NVLink flight after the producing lane computed it.  Costs 2x the (tiny) bytes on the wire.
+// ---- protocol A: every pushed value travels with its epoch in ONE 8-byte store {value bits, epoch32}:
+// the push is visible one NVLink flight after the producing lane computed it.  Costs 2x the (tiny)
+// bytes on the wire.
 __device__ __forceinline__ void st_peer_pair(void* p, float v, uint32_t epoch) {
   asm volatile("st.relaxed.sys.global.v2.u32 [%0], {%1,%2};" ::"l"(p), "r"(__float_as_uint(v)), "r"(epoch) : "memory");
 }
 __device__ __forceinline__ uint4 ld_pairs(const uint4* p) {   // two {value, epoch} pairs
   uint4 v;
   asm volatile("ld.relaxed.sys.global.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p) : "memory");
-  return v;
-}
-// the same pairs inside ONE GPU (the consumer grid's own all-gather of the folded residual): gpu scope
-__device__ __forceinline__ void st_pairs_gpu(uint4* p, float a, float b, uint32_t epoch) {
-  asm volatile("st.relaxed.gpu.global.v4.u32 [%0], {%1,%2,%3,%4};" ::"l"(p), "r"(__float_as_uint(a)), "r"(epoch), "r"(__float_as_uint(b)), "r"(epoch) : "memory");
-}
-__device__ __forceinline__ uint4 ld_pairs_gpu(const uint4* p) {
-  uint4 v;
-  asm volatile("ld.relaxed.gpu.global.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p) : "memory");
   return v;
 }
 __device__ __forceinline__ TpFlags* tp_flags(const TpCtx& c, uint32_t r) {
@@ -144,22 +135,6 @@ __device__ __forceinline__ float4 tp_take_pairs(TpFlags* mine, const uint4* p, u
     unsigned int spins = 0;
     do {
       a = ld_pairs(p); b = ld_pairs(p + 1);
-      if ((++spins & 0xFFFu) == 0 && gtime_ns() - t0 > 20000000000ull) {
-        mine->timed_out = 1;
-        __threadfence_system();
-        __trap();
-      }
-    } while (a.y != epoch || a.w != epoch || b.y != epoch || b.w != epoch);
-  }
-  return make_float4(__uint_as_float(a.x), __uint_as_float(a.z), __uint_as_float(b.x), __uint_as_float(b.z));
-}
-// same, for pairs written by other CTAs of this GPU
-__device__ __forceinline__ float4 tp_take_pairs_gpu(TpFlags* mine, const uint4* p, uint4 a, uint4 b, uint32_t epoch) {
-  if (a.y != epoch || a.w != epoch || b.y != epoch || b.w != epoch) {
-    const unsigned long long t0 = gtime_ns();
-    unsigned int spins = 0;
-    do {
-      a = ld_pairs_gpu(p); b = ld_pairs_gpu(p + 1);
       if ((++spins & 0xFFFu) == 0 && gtime_ns() - t0 > 20000000000ull) {
         mine->timed_out = 1;
         __threadfence_system();
@@ -242,8 +217,8 @@ __device__ __forceinline__ void tp_signal_when_grid_done(const TpCtx& c, unsigne
 size_t tp_region_prefix_bytes();      // ArSignals + TpFlags
 int tp_step_begin(const TpCtx& c, cudaStream_t st);
 // fallbacks of protocol A for projection shapes the fused GEMV does not take
-int tp_push_rows(const TpCtx& c, uint32_t coll, const float* partial, uint32_t rows, uint32_t hidden, bool ll, cudaStream_t st);
-int tp_fold_rows(const TpCtx& c, uint32_t coll, const float* x_in, float* x_out, uint32_t rows, uint32_t hidden, bool ll, cudaStream_t st);
+int tp_push_rows(const TpCtx& c, uint32_t coll, const float* partial, uint32_t rows, uint32_t hidden, cudaStream_t st);
+int tp_fold_rows(const TpCtx& c, uint32_t coll, const float* x_in, float* x_out, uint32_t rows, uint32_t hidden, cudaStream_t st);
 // protocol B consumer
 // wait_ag: the grid does not end before every owner's rows arrived here (for consumers of y that are
 // not tensor-core GEMMs; those wait for the flags themselves: TpPushRS::wait_coll_plus1)

@@ -189,9 +189,10 @@ tp_reduce_norm_kernel(TpCtx c, uint32_t coll, float* __restrict__ x, const __nv_
 }
 
 // ---------------------------------------------------------------- protocol A, unfused -------
-// partial [rows <= 4][hidden] fp32 (local) -> slot[coll & 1][src = me] of every rank, then flag
+// partial [rows <= 4][hidden] fp32 (local) -> {value, epoch} pairs in slot[coll & 1][src = me] of every rank.
+// A 16-byte store of two pairs is not one atomic unit, but each 8-byte pair is: enough.
 __global__ void __launch_bounds__(256)
-tp_push_rows_kernel(TpCtx c, uint32_t coll, const float* __restrict__ partial, uint32_t rows, uint32_t hidden, uint32_t ll) {
+tp_push_rows_kernel(TpCtx c, uint32_t coll, const float* __restrict__ partial, uint32_t rows, uint32_t hidden) {
   const uint32_t slot = coll & 1;
   const uint32_t n4 = rows * hidden / 4;
   const uint32_t h4 = hidden / 4;
@@ -199,49 +200,28 @@ tp_push_rows_kernel(TpCtx c, uint32_t coll, const float* __restrict__ partial, u
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += gridDim.x * blockDim.x) {
     const float4 v = reinterpret_cast<const float4*>(partial)[i];
     const uint32_t row = i / h4, col = i - row * h4;
-    if (ll) {   // {value, epoch} pairs, two 16-byte stores per float4
-      for (uint32_t r = 0; r < c.size; ++r) {
-        uint4* dst = reinterpret_cast<uint4*>(c.base[r] + c.ll_off[slot]) + ((size_t(c.rank) * kTpSmallRows + row) * hidden + 4 * size_t(col)) / 2;
-        asm volatile("st.relaxed.sys.global.v4.u32 [%0], {%1,%2,%3,%4};" ::"l"(dst), "r"(__float_as_uint(v.x)), "r"(ep32), "r"(__float_as_uint(v.y)), "r"(ep32) : "memory");
-        asm volatile("st.relaxed.sys.global.v4.u32 [%0], {%1,%2,%3,%4};" ::"l"(dst + 1), "r"(__float_as_uint(v.z)), "r"(ep32), "r"(__float_as_uint(v.w)), "r"(ep32) : "memory");
-      }
-      continue;
-    }
     for (uint32_t r = 0; r < c.size; ++r) {
-      float4* dst = reinterpret_cast<float4*>(c.base[r] + c.slot_off[slot]) +
-                    (size_t(c.rank) * kTpSmallRows + row) * h4 + col;
-      asm volatile("st.relaxed.sys.global.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(dst), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
+      uint4* dst = reinterpret_cast<uint4*>(c.base[r] + c.ll_off[slot]) + ((size_t(c.rank) * kTpSmallRows + row) * hidden + 4 * size_t(col)) / 2;
+      asm volatile("st.relaxed.sys.global.v4.u32 [%0], {%1,%2,%3,%4};" ::"l"(dst), "r"(__float_as_uint(v.x)), "r"(ep32), "r"(__float_as_uint(v.y)), "r"(ep32) : "memory");
+      asm volatile("st.relaxed.sys.global.v4.u32 [%0], {%1,%2,%3,%4};" ::"l"(dst + 1), "r"(__float_as_uint(v.z)), "r"(ep32), "r"(__float_as_uint(v.w)), "r"(ep32) : "memory");
     }
   }
-  if (ll) return;   // a 16-byte store of two pairs is not one atomic unit, but each 8-byte pair is: enough
-  TpFlags* mine = tp_flags(c, c.rank);
-  tp_signal_when_grid_done(c, &mine->done[slot], gridDim.x, tp_epoch(c, coll),
-                           [&](TpFlags* f) { return &f->push_flag[slot][c.rank]; });
 }
 // x_out = x_in + sum over src of slot[src]   (rows <= 4)
 __global__ void __launch_bounds__(256)
 tp_fold_rows_kernel(TpCtx c, uint32_t coll, const float* __restrict__ x_in, float* __restrict__ x_out,
-                    uint32_t rows, uint32_t hidden, uint32_t ll) {
+                    uint32_t rows, uint32_t hidden) {
   const uint32_t slot = coll & 1;
   TpFlags* mine = tp_flags(c, c.rank);
-  if (!ll) tp_wait_flags(mine, mine->push_flag[slot], c.size, tp_epoch(c, coll));
   const uint32_t ep32 = tp_epoch32(c, coll);
   const uint32_t n4 = rows * hidden / 4, h4 = hidden / 4;
-  const float4* sb = reinterpret_cast<const float4*>(c.base[c.rank] + (ll ? c.ll_off[slot] : c.slot_off[slot]));
+  const uint4* sb = reinterpret_cast<const uint4*>(c.base[c.rank] + c.ll_off[slot]);
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += gridDim.x * blockDim.x) {
     const uint32_t row = i / h4, col = i - row * h4;
     float4 v = reinterpret_cast<const float4*>(x_in)[i];
-    if (ll) {
-      for (uint32_t r = 0; r < c.size; ++r) {
-        const uint4* pp = reinterpret_cast<const uint4*>(sb) + ((size_t(r) * kTpSmallRows + row) * hidden + 4 * size_t(col)) / 2;
-        const float4 a = tp_take_pairs(mine, pp, ld_pairs(pp), ld_pairs(pp + 1), ep32);
-        v.x += a.x; v.y += a.y; v.z += a.z; v.w += a.w;
-      }
-      reinterpret_cast<float4*>(x_out)[i] = v;
-      continue;
-    }
     for (uint32_t r = 0; r < c.size; ++r) {
-      const float4 a = ld_pushed_f4(sb + (size_t(r) * kTpSmallRows + row) * h4 + col);
+      const uint4* pp = sb + ((size_t(r) * kTpSmallRows + row) * hidden + 4 * size_t(col)) / 2;
+      const float4 a = tp_take_pairs(mine, pp, ld_pairs(pp), ld_pairs(pp + 1), ep32);
       v.x += a.x; v.y += a.y; v.z += a.z; v.w += a.w;
     }
     reinterpret_cast<float4*>(x_out)[i] = v;
@@ -314,7 +294,7 @@ int tp_reduce_norm(const TpCtx& c, uint32_t coll, float* x, const void* gain, ui
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = (g_dbg_no_pdl & 16u) ? 0 : 1;
+  cfg.numAttrs = 1;
   if (ll)
     LLMLB_CUDA_CHECK(cudaLaunchKernelEx(&cfg, tp_reduce_norm_kernel<true>, c, coll, x, (const __nv_bfloat16*)gain, n_tokens, rpr, n_own,
                                         hidden, eps, c.size * split_k, wait_ag ? 1u : 0u));
@@ -325,17 +305,17 @@ int tp_reduce_norm(const TpCtx& c, uint32_t coll, float* x, const void* gain, ui
   return LLMLB_OK;
 }
 
-int tp_push_rows(const TpCtx& c, uint32_t coll, const float* partial, uint32_t rows, uint32_t hidden, bool ll, cudaStream_t st) {
+int tp_push_rows(const TpCtx& c, uint32_t coll, const float* partial, uint32_t rows, uint32_t hidden, cudaStream_t st) {
   uint32_t blocks = (rows * hidden / 4 + 255) / 256;
   if (blocks > 32) blocks = 32;
-  tp_push_rows_kernel<<<blocks, 256, 0, st>>>(c, coll, partial, rows, hidden, ll ? 1u : 0u);
+  tp_push_rows_kernel<<<blocks, 256, 0, st>>>(c, coll, partial, rows, hidden);
   LLMLB_LAUNCH_CHECK();
   return LLMLB_OK;
 }
-int tp_fold_rows(const TpCtx& c, uint32_t coll, const float* x_in, float* x_out, uint32_t rows, uint32_t hidden, bool ll, cudaStream_t st) {
+int tp_fold_rows(const TpCtx& c, uint32_t coll, const float* x_in, float* x_out, uint32_t rows, uint32_t hidden, cudaStream_t st) {
   uint32_t blocks = (rows * hidden / 4 + 255) / 256;
   if (blocks > 32) blocks = 32;
-  tp_fold_rows_kernel<<<blocks, 256, 0, st>>>(c, coll, x_in, x_out, rows, hidden, ll ? 1u : 0u);
+  tp_fold_rows_kernel<<<blocks, 256, 0, st>>>(c, coll, x_in, x_out, rows, hidden);
   LLMLB_LAUNCH_CHECK();
   return LLMLB_OK;
 }

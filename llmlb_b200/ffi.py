@@ -91,7 +91,6 @@ PROTOTYPES = {
     "llmlb_op_gemm": (C.c_int, [vp, vp, vp, u32, u32, u32, u32, u32, u32, vp]),
     "llmlb_op_rope_table": (C.c_int, [vp, u32, f32, vp]),
     "llmlb_op_rope_append": (C.c_int, [vp, vp, vp, vp, vp, vp, u32, u32, u32, vp]),
-    "llmlb_op_prefill_attention": (C.c_int, [vp, vp, vp, vp, u32, vp, u32, vp, u32, u32, vp]),
     "llmlb_op_prefill_attention_tc": (C.c_int, [vp, u32, vp, vp, u32, vp, u32, vp, u32, vp, u32, u32, vp]),
     "llmlb_op_decode_attention_ws": (C.c_size_t, [u32, u32, u32]),
     "llmlb_op_decode_attention": (C.c_int, [vp, vp, vp, vp, u32, vp, vp, u32, vp, u32, u32, vp,
@@ -157,7 +156,7 @@ class Engine:
 
     def __init__(self, model, model_id="llama-3-8b-synthetic", device=0, tp_rank=0, tp_size=1,
                  max_seqs=8, max_ctx=1024, kv_pages=0, max_step_tokens=0, seed=0,
-                 use_cuda_graphs=True, gemm_impl=0, lookahead=0, queue_max=0, queue_timeout_ms=0, request_timeout_ms=0, attn_impl=0, tp_proto=0):
+                 use_cuda_graphs=True, lookahead=0, queue_max=0, queue_timeout_ms=0, request_timeout_ms=0, tp_proto=0):
         cfg = EngineConfig()
         cfg.abi_version = ABI_VERSION
         for k, v in model.items():
@@ -168,9 +167,9 @@ class Engine:
         cfg.kv_pages, cfg.max_step_tokens = kv_pages, max_step_tokens
         cfg.synthetic_seed = seed
         cfg.use_cuda_graphs = 1 if use_cuda_graphs else 0
-        cfg.gemm_impl, cfg.lookahead = gemm_impl, lookahead
+        cfg.lookahead = lookahead
         cfg.queue_max, cfg.queue_timeout_ms, cfg.request_timeout_ms = queue_max, queue_timeout_ms, request_timeout_ms
-        cfg.attn_impl, cfg.tp_proto = attn_impl, tp_proto
+        cfg.tp_proto = tp_proto   # must be 0: the library refuses any other value at create
         self.model = dict(model)
         self.cfg = cfg
         self._h = vp()

@@ -43,7 +43,7 @@ def f():
 calls = crashes = 0
 hist = {}
 for _ in range(int(sys.argv[1])):
-    op = rs.randrange(12)
+    op = rs.randrange(11)
     if op == 0:
         rc = L.llmlb_op_embed(ptr(), ptr(), ptr(), u(), u(), u(), None)
     elif op == 1:
@@ -57,15 +57,13 @@ for _ in range(int(sys.argv[1])):
     elif op == 5:
         rc = L.llmlb_op_rope_append(ptr(), ptr(), ptr(), ptr(), ptr(), ptr(), u(), u(), u(), None)
     elif op == 6:
-        rc = L.llmlb_op_prefill_attention(ptr(), ptr(), ptr(), ptr(), u(), ptr(), u(), ptr(), u(), u(), None)
-    elif op == 7:
         rc = L.llmlb_op_prefill_attention_tc(ptr(), u(), ptr(), ptr(), u(), ptr(), u(), ptr(), u(), ptr(), u(), u(), None)
-    elif op == 8:
+    elif op == 7:
         L.llmlb_op_decode_attention_ws(u(), u(), u())
         rc = L.llmlb_op_decode_attention(ptr(), ptr(), ptr(), ptr(), u(), ptr(), ptr(), u(), ptr(), u(), u(), ptr(), u(), u(), ptr(), None)
-    elif op == 9:
+    elif op == 8:
         rc = L.llmlb_op_sample(ptr(), u(), u(), ptr(), ptr(), ptr(), ptr(), ptr(), ptr(), None)
-    elif op == 10:
+    elif op == 9:
         rc = L.llmlb_op_synth_bf16(ptr(), u(), u(), u(), u(), u(), u(), rs.randrange(40), f(), None)
     else:
         rc = L.llmlb_op_allreduce(None, ptr(), u(), None)

@@ -15,12 +15,12 @@ def header_functions():
     return sorted(set(re.findall(r"\b(llmlb_[a-z0-9_]+)\s*\(", src)))
 
 
-def test_header_declares_expected_surface():
+def test_header_declares_the_engine_and_kernel_entry_points():
     fns = header_functions()
     for must in ["llmlb_engine_create", "llmlb_engine_destroy", "llmlb_request_submit",
                  "llmlb_request_poll", "llmlb_request_cancel", "llmlb_engine_health",
                  "llmlb_engine_model_info", "llmlb_last_error", "llmlb_op_gemv", "llmlb_op_gemm",
-                 "llmlb_op_decode_attention", "llmlb_op_prefill_attention", "llmlb_op_sample"]:
+                 "llmlb_op_decode_attention", "llmlb_op_prefill_attention_tc", "llmlb_op_sample"]:
         assert must in fns
 
 

@@ -739,3 +739,24 @@ def test_scenario_tensor_parallel_depth_limit_is_refused_not_wrapped():
         ffi.Engine(dict(ffi.LLAMA3_70B, n_layers=128), tp_size=8, tp_rank=0, max_seqs=2, max_ctx=256)
     assert "127 layers" in str(ei.value)
     ffi.Engine(dict(TINY, n_layers=200), max_seqs=2, max_ctx=256).close()
+
+
+@inner
+@pytest.mark.parametrize("field,value", [("attn_impl", 1), ("tp_proto", 1), ("tp_proto", 2)])
+def test_scenario_implementation_switches_other_than_zero_are_refused_at_create(field, value):
+    """gemm_impl, attn_impl and tp_proto keep their places in the config struct, but the library holds one implementation
+    of each: any value other than 0 is refused at create, not ignored.  The same config with 0 creates an engine."""
+    import ctypes as C
+    ffi = _ffi()
+    cfg = ffi.EngineConfig()
+    cfg.abi_version = ffi.ABI_VERSION
+    for k, v in TINY.items():
+        setattr(cfg.model, k, v)
+    cfg.max_seqs, cfg.max_ctx, cfg.kv_block_tokens = 2, 256, 64
+    setattr(cfg, field, value)
+    h = C.c_void_p()
+    assert ffi.lib().llmlb_engine_create(C.byref(cfg), C.byref(h)) == ffi.E_INVALID_ARG and not h
+    assert field in ffi.last_error()
+    setattr(cfg, field, 0)
+    assert ffi.lib().llmlb_engine_create(C.byref(cfg), C.byref(h)) == ffi.OK and h
+    ffi.lib().llmlb_engine_destroy(h)

@@ -3,8 +3,8 @@ CUDA runtime and logs every kernel launch for EVERY prefill width 1..2048 and de
 (tp 1, 2, 4, 8) and Llama-3-70B (tp 8) shapes.  Checked on each launch:
 
   * co-residency: kernels whose CTAs wait for each other inside the grid (the in-kernel K-split of gemm_tc / gemm_tc2 parks
-    partial tiles and spins on a per-tile counter; the gemv_ks gather variant waits for owner CTAs) must fit the GPU in one
-    wave — at most 148 CTAs at one CTA per SM.  A wider grid would hang the device; GPU tests only ever try a few widths.
+    partial tiles and spins on a per-tile counter) must fit the GPU in one wave — at most 148 CTAs at one CTA per SM; gemv_ks
+    is held to the same bound.  A wider grid would hang the device; GPU tests only ever try a few widths.
   * hardware limits: <= 1024 threads per CTA, <= 227 KiB dynamic shared memory, cluster size <= 16 and grid divisible by it.
   * every launch with more than 48 KiB of dynamic shared memory was preceded by the opt-in for THAT kernel function (each
     template instantiation needs its own cudaFuncSetAttribute; a missing one only fails at the widths that pick it) — the
@@ -128,7 +128,7 @@ def test_op_gemm_accepts_arbitrary_shapes_within_the_same_limits(built_lib, tmp_
     assert calls > 5000 and launches >= calls
 
 
-def test_kernel_level_entry_points_survive_random_arguments(built_lib, tmp_path):
+def test_every_kernel_level_entry_point_survives_random_arguments(built_lib, tmp_path):
     """Every llmlb_op_* entry point with random pointers (valid or NULL) and integers from {0, 1, odd, model-sized, 2^32 - 1}:
     25000 calls, each returns OK or a negative error code — never a crash.  Found on the first run: a dimension near 2^32
     wrapped llmlb_op_gemm's 32-bit tile count to zero and the launch planner divided by it (SIGFPE); dimensions are

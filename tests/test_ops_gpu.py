@@ -182,10 +182,10 @@ def test_rope_table(L):
     assert torch.allclose(tab[..., 1].cpu().double(), torch.sin(ang), atol=1e-6)
 
 
-def _prefill_attention_case(L, nh, nkv, seqs, impl):
-    """Sequences packed in one step (ragged; some with earlier context already in the cache) against
-    dense fp32 attention.  seqs: list of (context tokens already cached, new tokens).
-    impl "mma": llmlb_op_prefill_attention, 64-row tiles; "tc": the tcgen05 kernel, 128-row tiles."""
+def _prefill_attention_case(L, nh, nkv, seqs):
+    """Sequences packed in one step (ragged; some with earlier context already in the cache) through
+    llmlb_op_prefill_attention_tc (128-row q tiles) against dense fp32 attention.
+    seqs: list of (context tokens already cached, new tokens)."""
     torch.manual_seed(0)
     max_len = max(c + n for c, n in seqs)
     rope = _mk_rope(L, 2048)
@@ -212,7 +212,7 @@ def _prefill_attention_case(L, nh, nkv, seqs, impl):
     pos = torch.cat([torch.arange(c, c + n) for c, n in seqs]).to(torch.int32).to(dev())
     page = torch.cat([bt[i][(torch.arange(c, c + n) // 64).long().to(dev())] for i, (c, n) in enumerate(seqs)]).contiguous()
     ok(L.llmlb_op_rope_append(p(qkv), p(pos), p(page), p(rope), p(kp), p(vp), T, nh, nkv, stream_ptr()))
-    tile = 64 if impl == "mma" else 128
+    tile = 128
     tiles, row0 = [], 0
     for i, (c, n) in enumerate(seqs):
         for j in range(0, n, tile):
@@ -220,11 +220,8 @@ def _prefill_attention_case(L, nh, nkv, seqs, impl):
         row0 += n
     tiles_t = torch.tensor(tiles, dtype=torch.int32, device=dev())
     out = torch.zeros(T, nh * 128, dtype=torch.bfloat16, device=dev())
-    if impl == "mma":
-        ok(L.llmlb_op_prefill_attention(p(qkv), p(kp), p(vp), p(bt), bt_stride, p(tiles_t), len(tiles), p(out), nh, nkv, stream_ptr()))
-    else:
-        ok(L.llmlb_op_prefill_attention_tc(p(qkv), T, p(kp), p(vp), n_pages, p(bt), bt_stride, p(tiles_t), len(tiles), p(out), nh, nkv,
-                                           stream_ptr()))
+    ok(L.llmlb_op_prefill_attention_tc(p(qkv), T, p(kp), p(vp), n_pages, p(bt), bt_stride, p(tiles_t), len(tiles), p(out), nh, nkv,
+                                       stream_ptr()))
     sync()
 
     def split(t):
@@ -257,10 +254,10 @@ def _prefill_attention_case(L, nh, nkv, seqs, impl):
 
 
 @pytest.mark.parametrize("nh,nkv", [(32, 8), (8, 2), (8, 1)])
-def test_rope_append_and_prefill_attention(L, nh, nkv):
+def test_rope_append_then_tcgen05_prefill_attention(L, nh, nkv):
     """Two sequences packed in one step (ragged: 150 and 37 tokens, the 2nd with 70 tokens of
     earlier context); also checks the rotated q / appended K,V bit patterns."""
-    raw, qkv, kp, vp, bt, rt, split = _prefill_attention_case(L, nh, nkv, [(0, 150), (70, 37)], "mma")
+    raw, qkv, kp, vp, bt, rt, split = _prefill_attention_case(L, nh, nkv, [(0, 150), (70, 37)])
     q0, k0, _ = split(raw[:150])
     # q,k rotated values in the activation buffer are bit-identical to the bf16-rounded reference
     assert torch.allclose(qkv[:, : nh * 128].float().view(-1, nh, 128)[:150], rt(q0, torch.arange(150, device=dev())), atol=1e-2, rtol=2 ** -7)
@@ -277,7 +274,7 @@ def test_prefill_attention_tcgen05(L, nh, nkv, seqs):
     consumed MN-major from its pages.  Edge cases: a 1-token prompt, exact page and block boundaries,
     a tile that starts in the middle of a page, contexts of several blocks, a block whose second
     page does not exist."""
-    _prefill_attention_case(L, nh, nkv, seqs, "tc")
+    _prefill_attention_case(L, nh, nkv, seqs)
 
 
 @pytest.mark.parametrize("nh,nkv", [(32, 8), (8, 2), (8, 1)])

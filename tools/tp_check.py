@@ -46,13 +46,12 @@ def geometry(world, kind):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--geom", default="tiny", choices=["tiny", "odd", "8b4"])
-    ap.add_argument("--proto", type=int, default=0, help="decode exchange: bit 0: 0 = {value, epoch} pairs, 1 = values + flags; bit 1: owner-fold + gather consumer")
     args = ap.parse_args()
     rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
     torch.cuda.set_device(local)
     dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     cfg = geometry(world, args.geom)
-    eng = ffi.Engine(cfg, device=local, tp_rank=rank, tp_size=world, max_seqs=8, max_ctx=1024, seed=0, tp_proto=args.proto)
+    eng = ffi.Engine(cfg, device=local, tp_rank=rank, tp_size=world, max_seqs=8, max_ctx=1024, seed=0)
     handles = [None] * world
     dist.all_gather_object(handles, eng.tp_export())
     eng.tp_import(handles)
@@ -117,9 +116,9 @@ def main():
         same = all(g == gathered[0] for g in gathered)
         eq3 = sum(int(a == b) for a, b in zip(toks3, ref3))
         lens_ok = all(len(t) == 24 for t in toks3) and all(len(t) == 10 for t in toks7)
-        print("tp=%d geom=8b4 proto=%d max|dlogit| vs tp=1 engine: prefill512 %.4g decode %.4g %.4g prefill3 %.4g decode %.4g (logit std %.3f); "
+        print("tp=%d geom=8b4 max|dlogit| vs tp=1 engine: prefill512 %.4g decode %.4g %.4g prefill3 %.4g decode %.4g (logit std %.3f); "
               "ranks identical: %s; staggered requests token-identical to tp=1: %d/3; worst margin of a batched-step token to the tp=1 arg-max %.4f; lengths ok: %s"
-              % (world, args.proto, d[0], d[1], d[2], d[3], d[4], float(l1.std()), same, eq3, worst, lens_ok))
+              % (world, d[0], d[1], d[2], d[3], d[4], float(l1.std()), same, eq3, worst, lens_ok))
         # measured on B200: 0.062 (tp=2), 0.072 (tp=8) on prefill512 at a logit std of 1.28 (bf16 partials on the wire, N-way order)
         ok = max(d) < 0.10 and same and lens_ok and worst < 0.2
     elif rank == 0:
@@ -160,9 +159,9 @@ def main():
             s1 = [one.debug_decode_logits(7), one.debug_decode_logits(99)]
         d0 = float(np.abs(lg - l1).max())
         d1 = max(float(np.abs(a - b).max()) for a, b in zip(step, s1))
-        print("tp=%d geom=%s proto=%d max|dlogit| vs oracle: prefill150 %.4g decode %.4g %.4g prefill3 %.4g decode %.4g; vs tp=1 engine: prefill %.4g decode %.4g; "
+        print("tp=%d geom=%s max|dlogit| vs oracle: prefill150 %.4g decode %.4g %.4g prefill3 %.4g decode %.4g; vs tp=1 engine: prefill %.4g decode %.4g; "
               "ranks identical: %s; top-1 agreement %d/%d (per request %s), all near-argmax: %s, lengths ok: %s"
-              % (world, args.geom, args.proto, e0, e1, e2, e3, e4, d0, d1, same, agree, total, " ".join(detail), near, lens_ok))
+              % (world, args.geom, e0, e1, e2, e3, e4, d0, d1, same, agree, total, " ".join(detail), near, lens_ok))
         ok = max(e0, e1, e2, e3, e4) < TOL and max(d0, d1) < TOL and same and near and lens_ok and agree >= int(0.9 * total)
     flag = torch.tensor([1 if ok else 0], device="cuda")
     dist.broadcast(flag, 0)

@@ -23,7 +23,6 @@ from llmlb_b200 import ffi  # noqa: E402
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--max-seqs", type=int, default=64)
-    ap.add_argument("--proto", type=int, default=0)
     ap.add_argument("--lookahead", type=int, default=0)
     ap.add_argument("--no-graphs", action="store_true")
     ap.add_argument("--runs", type=int, default=4)
@@ -36,7 +35,7 @@ def main():
     dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     model = ffi.LLAMA3_8B
     eng = ffi.Engine(model, device=local, tp_rank=rank, tp_size=world, max_seqs=args.max_seqs, max_ctx=1024, seed=0,
-                     kv_pages=args.kv_pages, use_cuda_graphs=not args.no_graphs, lookahead=args.lookahead, tp_proto=args.proto)
+                     kv_pages=args.kv_pages, use_cuda_graphs=not args.no_graphs, lookahead=args.lookahead)
     handles = [None] * world
     dist.all_gather_object(handles, eng.tp_export())
     eng.tp_import(handles)
@@ -78,9 +77,9 @@ def main():
                 if i + 1 < len(seqs[0]):
                     lg = one.debug_decode_logits(t)
         worst = int(np.argmax(m1))
-        print("%s tp=%d max_seqs=%d proto=%d graphs=%s lookahead=%d: %d distinct sequences in %d runs (first divergence %s), ranks identical %s | "
+        print("%s tp=%d max_seqs=%d graphs=%s lookahead=%d: %d distinct sequences in %d runs (first divergence %s), ranks identical %s | "
               "vs own eager path: top-1 %d/%d, max margin %.4f at step %d | vs tp=1 engine: top-1 %d/%d, max margin %.4f at step %d, margins > 0.1 at steps %s"
-              % (args.tag, world, args.max_seqs, args.proto, not args.no_graphs, args.lookahead or 2, len(set(map(tuple, seqs))), len(seqs), first_div,
+              % (args.tag, world, args.max_seqs, not args.no_graphs, args.lookahead or 2, len(set(map(tuple, seqs))), len(seqs), first_div,
                  all(a == seqs for a in allr), own_agree, len(own_m), max(own_m), int(np.argmax(own_m)), agree1, len(m1), max(m1), worst,
                  [i for i, v in enumerate(m1) if v > 0.1]))
         sys.stdout.flush()

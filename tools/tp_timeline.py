@@ -86,9 +86,9 @@ def report(title, ls, detail_rows=None, max_lines=16):
         print("%-34s %4d %10.1f %12.1f %12.1f" % (k, d["n"], d["span"], d["after_dep"], d["exposed"]))
     if detail_rows is not None and len(detail_rows):
         a = detail_rows.astype(np.int64)
-        w = (a[:, 3] - a[:, 2]) / 1e3   # dependency satisfied -> flags in
-        f = (a[:, 4] - a[:, 3]) / 1e3   # flags in -> fold + norm done
-        print("GEMV consumers (protocol A): wait for the push flags after the local dependency: mean %.2f us, p95 %.2f, max %.2f; fold + norm: mean %.2f us"
+        w = (a[:, 3] - a[:, 2]) / 1e3   # dependency satisfied -> every peer's pairs arrived and folded
+        f = (a[:, 4] - a[:, 3]) / 1e3   # fold done -> norm done
+        print("GEMV consumers (protocol A): wait for + fold of the pushed pairs after the local dependency: mean %.2f us, p95 %.2f, max %.2f; norm: mean %.2f us"
               % (w.mean(), np.percentile(w, 95), w.max(), f.mean()))
 
 
@@ -96,7 +96,6 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--streams", type=int, default=1)
     ap.add_argument("--gen", type=int, default=6)
-    ap.add_argument("--proto", type=int, default=0)
     args = ap.parse_args()
     rank, world, local = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("LOCAL_RANK", 0))
     dist = None
@@ -109,7 +108,7 @@ def main():
     L.llmlb_debug_trace_enable.argtypes = [C.c_uint32]
     L.llmlb_debug_trace_dump.argtypes = [C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32)]
     model = ffi.LLAMA3_8B
-    eng = ffi.Engine(model, device=local, tp_rank=rank, tp_size=world, max_seqs=max(4, args.streams), max_ctx=1024, seed=0, tp_proto=args.proto)
+    eng = ffi.Engine(model, device=local, tp_rank=rank, tp_size=world, max_seqs=max(4, args.streams), max_ctx=1024, seed=0)
     if world > 1:
         handles = [None] * world
         dist.all_gather_object(handles, eng.tp_export())
